@@ -2,7 +2,7 @@
 """bench.py -- co-occurrence updates/sec of the GloVe TRAIN step on B200 (metric of BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload wiki6b|text8|cc|topk]
-                    [--adam-mode replay|replay_exact|lazy|dense]
+                    [--adam-mode replay|replay_exact|lazy|dense] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference path's CPU restatement on the box's host cores
 
@@ -190,6 +190,43 @@ def cpu_reference(V, d, B, steps, warmup, seed=0):
     return steps * B / dt, dt, c_oracle.num_threads()
 
 
+DUMP_HEAD, DUMP_SAMPLE = 4096, 12288   # rows dumped per table: the most frequent ids + a seeded sample of the rest
+DUMP_LIMIT = 64 << 20                  # bytes
+
+
+def train_outputs(eng, losses):
+    """What a caller of the TRAIN step holds after the last timed step: the losses of the timed steps and the variables in
+    reference layout (lazy Adam state replayed up to the current step, as GloveEngine.get_state gives them), on a fixed
+    set of rows: ids 0 .. DUMP_HEAD-1 (Zipf head: touched by nearly every step) and a seeded sample of the others."""
+    import torch
+    V = eng.V
+    rows = np.arange(V)
+    if V > DUMP_HEAD + DUMP_SAMPLE:
+        tail = np.random.default_rng(0).choice(np.arange(DUMP_HEAD, V), DUMP_SAMPLE, replace=False)
+        rows = np.concatenate([rows[:DUMP_HEAD], np.sort(tail)])
+    eng.flush()
+    idx = torch.from_numpy(rows).to(eng.device)
+    out = {"losses": losses, "rows": rows}
+    for name, bname, table in (("R", "rb", eng.row_table), ("C", "cb", eng.col_table)):
+        e, b = eng._unpack(table, 0)
+        out[name], out[bname] = e[idx].cpu().numpy(), b[idx].cpu().numpy()
+        del e, b
+    out["g"] = np.array([eng.read_scalars()["g"]], np.float32)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """<out_dir>/<name>.npy for every array: float32 stays float32, anything else (ids included, exactly) is float64."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def load_traffic(key):
     """(bytes per step, source) from profiles/step_traffic.json: {key: {"dram_bytes": n, "source": "profiles/..."}}."""
     try:
@@ -199,16 +236,17 @@ def load_traffic(key):
         return None, None
 
 
-def topk_record(dev, sampler, full_line=False, n_gpus=1, steps=5, warmup=3):
+def topk_record(dev, sampler, full_line=False, n_gpus=1, steps=5, warmup=3, outputs=None):
     """BASELINE configs[4]: cosine top-k of Q = 65,536 query rows over a 2.2M x 300 table, k = 10 (tcgen05 candidate pass +
     exact fp32 re-score), per GPU (N > 1: replicas, queries sharded -- every rank runs the same call).  Algorithmic flops
     = 2*Q*V*d (padding d to 320 is overhead, not credit).  `value` is device-timed (CUDA events around the whole topk
     call incl. normalised-query gather, candidate pass, re-score, guarantee check; query ids resident); `e2e` is the wall
-    time of GloveEngine.topk from HOST query ids to HOST results."""
+    time of GloveEngine.topk from HOST query ids to HOST results.  `outputs` (a dict) receives the last timed call's
+    results as topk_sim / topk_idx [Q, k]."""
     import torch
     from glove_tensorflow_b200.engine import GloveEngine
     V, d, Q, k = TOPK
-    iters = max(1, min(steps, 10))
+    iters = max(1, steps)
     eng = GloveEngine(V, d, optimizer="SGD", batch_size=64, plan_steps=1, max_steps=4, device=dev)
     eng.init_uniform(0)
     q = torch.randint(0, V, (Q,), generator=torch.Generator().manual_seed(1)).numpy().astype(np.int32)
@@ -221,11 +259,13 @@ def topk_record(dev, sampler, full_line=False, n_gpus=1, steps=5, warmup=3):
     inv, nb = eng._normalised_table()
     ev[0].record()
     for _ in range(iters):
-        eng._topk_call(inv, nb, eng.row_table, eng.P, nb, qd, Q, k, False)
+        sim, idx = eng._topk_call(inv, nb, eng.row_table, eng.P, nb, qd, Q, k, False)
     ev[1].record()
     torch.cuda.synchronize()
     ms = ev[0].elapsed_time(ev[1]) / iters
     fallbacks = eng.last_topk_fallbacks
+    if outputs is not None:
+        outputs["topk_sim"], outputs["topk_idx"] = sim.cpu().numpy().reshape(Q, k), idx.cpu().numpy().reshape(Q, k)
     t0 = time.perf_counter()
     for _ in range(iters):
         eng.topk(q, k)
@@ -320,7 +360,14 @@ def main():
                          "kernel over NVLink peer memory; falls back to alltoall when symmetric memory is unavailable)")
     ap.add_argument("--dp-mode", default="sharded", choices=["sharded", "replicated"],
                     help="N>1: row-sharded tables (owner-computes) or replicated tables with gradient all-reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (a fixed sample of the "
+                         "tables; with --workload topk or the default run's topk record, the top-k results too)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl b200 on one GPU")
 
     V, d, B_local, nnz = WORKLOADS["wiki6b" if args.workload == "topk" else args.workload]
     B_local = args.batch or B_local
@@ -386,10 +433,14 @@ def main():
         sampler.start()
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
+    outputs = {} if args.dump_outputs else None
     if args.workload == "topk":
-        line = topk_record(dev, sampler if rank == 0 else None, full_line=True, n_gpus=N, steps=args.steps, warmup=args.warmup)
+        line = topk_record(dev, sampler if rank == 0 else None, full_line=True, n_gpus=N, steps=args.steps, warmup=args.warmup,
+                           outputs=outputs)
         if rank == 0:
             sampler.stop()
+            if outputs is not None:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps(line))
         if world > 1:
             dist.destroy_process_group()
@@ -481,6 +532,8 @@ def main():
     assert np.all(np.isfinite(losses)), "non-finite loss in the timed region"
     value = B * args.steps / (ms * 1e-3)
     final_loss = losses[-1]
+    if outputs is not None:
+        outputs.update(train_outputs(eng, losses))
 
     # ---- roofline: per-kernel durations (CUDA events on the launching stream) + algorithmic bytes -------------------
     U = np.array([eng.batch_counts(s)[:2] for s in range(first_timed, first_timed + min(args.steps, 32))], np.float64)
@@ -591,8 +644,10 @@ def main():
     if N == 1 and not args.no_topk and args.workload == "wiki6b":
         eng = row = col = tgt = wgt = None                 # free the training state before the 2.2M-row table
         torch.cuda.empty_cache()
-        topk = topk_record(dev, sampler)
+        topk = topk_record(dev, sampler, outputs=outputs)
     sampler.stop()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     cpu = None
     if not args.no_cpu_baseline and N == 1:
