@@ -31,7 +31,17 @@ constexpr int TC_MAX_KCH = 5;  // Kp <= 320
 constexpr uint32_t TC_A_HALF_BYTES = TC_M * TC_KC * 2;    // 16 KB
 constexpr uint32_t TC_A_CHUNK_BYTES = TC_MQ * TC_KC * 2;  // 32 KB: rows 0-127 then rows 128-255
 constexpr uint32_t TC_B_STAGE_BYTES = TC_N * TC_KC * 2;   // 16 KB
-constexpr float TC_DELTA = 4.0e-3f;  // bound on |bf16 similarity - fp32 similarity| for unit vectors (2^-8 + slack)
+// Bound on |bf16 MMA similarity - fp32 similarity| of two rows normalised in fp32 (the guarantee check of rescore_kernel):
+//  * bf16 keeps 8 significant bits, so rounding to nearest moves each factor by up to 2^-8 of itself, and a product of
+//    two rounded factors by up to (1 + 2^-8)^2 - 1 = 2^-7 + 2^-16 of |q_c t_c|.  Summed over the columns, with
+//    sum |q_c t_c| <= |q| |t| (Cauchy-Schwarz), that is 7.83e-3 for unit vectors.  The bound is attained when every
+//    component sits just below a rounding midpoint (tests/test_topk_bound.py builds such a table): 2^-8 is NOT enough.
+//  * fp32 normalisation: the sum of squares is at most ~15 roundings deep (per-lane sum + butterfly), so |q|, |t| are
+//    within ~1e-6 of 1 -- a negligible change of the term above.
+//  * fp32 accumulation of the MMA and of cos_dot, Kp <= 320 products each: n u sum |q_c t_c| <= 320 * 2^-24 = 1.9e-5
+//    per sum with IEEE rounding; allowing twice that for the tensor core's own accumulation order, 6e-5 for both.
+// 7.83e-3 + 6e-5 < 7.9e-3; rounded up to 8e-3.
+constexpr float TC_DELTA = 8.0e-3f;
 
 // ---- PTX wrappers ----------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }

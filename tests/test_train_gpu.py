@@ -342,13 +342,17 @@ def test_row_sharded_tables_on_one_gpu(world, adam_mode, optimizer, V, exchange)
     """cfg4 scheme (SURVEY 8e): tables split row-wise over `world` owners (id % world), emulated as `world` engines on one
     GPU with the two collectives (all-gather of the owners' snapshot blocks, all-reduce of the loss scalars) done by
     hand; every owner runs the fused update of its own segments.  The union of the shards must match the single-process oracle."""
+    _run_row_sharded(world, adam_mode, optimizer, V, exchange)
+
+
+def _run_row_sharded(world, adam_mode, optimizer, V, exchange, d=40):
     import torch
     from glove_tensorflow_b200.engine import GloveEngine
     # "+shared-plans": the plan of chunk c is built by engine c % world alone and every engine copies its slice out of the
     # builder's buffer (glove_plan_pull_slice) -- results must not change by a bit (compared with the oracle like the rest)
     shared = exchange.endswith("+shared-plans")
     exchange = exchange.split("+")[0]
-    d, B, steps, n = 40, 512 if world != 3 else 510, 14, 20000
+    B, steps, n = 512 if world != 3 else 510, 14, 20000
     coo = make_coo(V, n, 51, hot=0.1)
     batches = np.random.default_rng(52).integers(0, n, (steps, B))
     st = o.init_state(V, d, 53)
