@@ -16,6 +16,7 @@ OPTIMIZERS = {"Adam": 0, "Adagrad": 1, "SGD": 2}
 # dense sweep's fp32 operations; "dense" = replay_exact + flush after every step (the literal legacy-Keras schedule)
 ADAM_MODES = {"replay": 0, "lazy": 1, "replay_exact": 2, "dense": 2}
 ABI_VERSION = 2
+ANALOGY_METHODS = {"add": 0, "mul": 1}   # 3CosAdd, 3CosMul (glove_analogy_topk)
 
 c_i32, c_i64, c_u32, c_f32 = ctypes.c_int32, ctypes.c_int64, ctypes.c_uint32, ctypes.c_float
 c_void, c_size = ctypes.c_void_p, ctypes.c_size_t
@@ -107,6 +108,10 @@ SIGNATURES = {
     "glove_topk_flagged": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_i32, ctypes.POINTER(c_i32), c_void]),
     "glove_topk_cosine_fp32": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_void, c_void, c_i32, c_i32, c_void,
                                               c_void, c_void, c_size, c_void]),
+    "glove_analogy_workspace_bytes": (c_size, [c_i64, c_i32, c_i32, c_i32, c_i32]),
+    "glove_analogy_topk": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_void, c_void, c_void, c_i32, c_i32, c_i32, c_void,
+                                          c_void, c_void, c_size, c_void]),
+    "glove_pair_cosine": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_void, c_void, c_i32, c_void, c_void]),
     "glove_vocab_slots": (c_i64, [c_i64]),
     "glove_vocab_build": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_i64, c_void]),
     "glove_csv_workspace_bytes": (c_size, [c_i64]),

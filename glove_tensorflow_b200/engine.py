@@ -1216,6 +1216,62 @@ class GloveEngine:
         torch.cuda.synchronize()
         return sim.cpu().numpy().reshape(n, k), idx.cpu().numpy().reshape(n, k)
 
+    # ---- intrinsic evaluation (evaluate_embeddings) ----------------------------------------------------------------
+    def _single_table(self, what):
+        if self.sharded:
+            raise RuntimeError("%s needs the whole row table on one GPU: load the checkpoint into a one-GPU engine "
+                               "(row-sharded engines are not evaluated in place)" % what)
+
+    def analogy(self, abc, k: int = 1, method: str = "add", restrict: Optional[int] = None, exact_fp32: bool = False):
+        """Word analogies a : b :: c : ? over the row table (glove_analogy_topk).  ``abc`` int [n, 3]; ``method`` "add"
+        (3CosAdd) or "mul" (3CosMul); the candidates are the first ``restrict`` rows (default all), a, b and c excluded.
+        Returns (score [n,k] f32, idx [n,k] i32) as numpy, scores descending, ties -> lower id.  ``exact_fp32`` makes
+        3CosAdd skip the tensor-core candidate pass (3CosMul is always an exact fp32 scan)."""
+        self._single_table("analogy")
+        if method not in _lib.ANALOGY_METHODS:
+            raise ValueError("analogy: method must be one of %s, not %r" % (sorted(_lib.ANALOGY_METHODS), method))
+        V = self.V if restrict is None else int(restrict)
+        if not 1 <= V <= self.V:
+            raise ValueError("analogy: restrict=%d not in [1, %d]" % (V, self.V))
+        abc = np.ascontiguousarray(abc, np.int64).reshape(-1, 3)
+        n = abc.shape[0]
+        if n == 0:
+            return np.zeros((0, k), np.float32), np.zeros((0, k), np.int32)
+        if abc.min() < 0 or abc.max() >= V:     # the kernels index the table with these: refuse, never clamp
+            raise ValueError("analogy: word ids must lie in [0, %d): min %d, max %d" % (V, abc.min(), abc.max()))
+        self.flush()
+        inv, nb = self._normalised_table()
+        m = _lib.ANALOGY_METHODS[method]
+        q = torch.as_tensor(abc.astype(np.int32)).to(self.device)
+        score = torch.empty(n * k, dtype=torch.float32, device=self.device)
+        idx = torch.empty(n * k, dtype=torch.int32, device=self.device)
+        ws = torch.empty(max(lib.glove_analogy_workspace_bytes(V, self.d, n, k, m), 256), dtype=torch.uint8, device=self.device)
+        use_tc = method == "add" and not exact_fp32
+        check(lib.glove_analogy_topk(_ptr(self.row_table), V, self.d, self.P, _ptr(nb) if use_tc else None, _ptr(inv),
+                                     _ptr(q), n, m, k, _ptr(score), _ptr(idx), _ptr(ws), ws.numel(), _stream()),
+              "glove_analogy_topk")
+        torch.cuda.synchronize()
+        return score.cpu().numpy().reshape(n, k), idx.cpu().numpy().reshape(n, k)
+
+    def pair_cosine(self, pairs) -> np.ndarray:
+        """Cosine of the row embeddings of each pair (int [n, 2]) as numpy f32 [n]: bit for bit the similarity that
+        ``topk([w1])`` reports for w2."""
+        self._single_table("pair_cosine")
+        pairs = np.ascontiguousarray(pairs, np.int64).reshape(-1, 2)
+        n = pairs.shape[0]
+        if n == 0:
+            return np.zeros(0, np.float32)
+        if pairs.min() < 0 or pairs.max() >= self.V:
+            raise ValueError("pair_cosine: word ids must lie in [0, %d): min %d, max %d" % (self.V, pairs.min(), pairs.max()))
+        self.flush()
+        inv, _ = self._normalised_table()
+        p = torch.as_tensor(pairs.astype(np.int32)).to(self.device)
+        out = torch.empty(n, dtype=torch.float32, device=self.device)
+        check(lib.glove_pair_cosine(_ptr(self.row_table), self.V, self.d, self.P, _ptr(inv), _ptr(p), n, _ptr(out), _stream()),
+              "glove_pair_cosine")
+        torch.cuda.synchronize()
+        return out.cpu().numpy()
+
     def tc_path_covers(self, k: int) -> bool:
         """Shapes the tcgen05 candidate pass handles (everything else runs the exact fp32 scan)."""
         return lib.glove_topk_kpad(self.d) <= 320 and k <= 24 and self.V >= 1024

@@ -23,3 +23,24 @@ def get_predictions(engine, input_ids, vocab, top_k=20):
         "top_k_similarity": sim,
         "top_k_string": [lookup(r) for r in idx],
     }
+
+
+def get_analogies(engine, triples, vocab, top_k=1, method="add"):
+    """Word analogies a : b :: c : ? for string triples (a, b, c): the ``top_k`` best rows outside {a, b, c} by 3CosAdd
+    (``method="add"``) or 3CosMul (``"mul"``).  Words are looked up exactly in ``vocab`` (the first line holding a token
+    wins); an unknown word raises KeyError.  Returns input_strings, top_k_score, top_k_string."""
+    first = {}
+    for i, tok in enumerate(vocab):
+        first.setdefault(tok, i)
+    triples = [tuple(t) for t in triples]
+    missing = sorted({w for t in triples for w in t if w not in first})
+    if missing:
+        raise KeyError("get_analogies: not in the vocabulary: %s" % ", ".join(missing[:10]))
+    abc = np.array([[first[w] for w in t] for t in triples], np.int64).reshape(-1, 3)
+    score, idx = engine.analogy(abc, top_k, method)
+    lookup = get_id_string_table(vocab)
+    return {
+        "input_strings": [list(t) for t in triples],
+        "top_k_score": score,
+        "top_k_string": [lookup(r) for r in idx],
+    }

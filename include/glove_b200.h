@@ -300,6 +300,30 @@ int glove_topk_cosine_fp32(const float *table, int64_t V, int32_t d, int32_t pla
                            const int32_t *query_ids, int32_t n_queries, int32_t k, float *out_sim, int32_t *out_idx,
                            void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---- Intrinsic evaluation: word analogies and word-pair similarity over the row table --------------------------------
+ * Conventions of Stanford GloVe eval/python/evaluate.py: rows are l2-normalised (here with the 1e-12 floor of
+ * tf.math.l2_normalize, as the top-k), the question (a, b, c) -> d is answered by the best row outside {a, b, c} (only
+ * those ids are excluded: a duplicate row of b under another id stays a candidate), ties -> lower id.
+ *   GLOVE_ANALOGY_ADD (3CosAdd): cosine of x with q = b^ - a^ + c^, ranked by the cosine top-k (tensor-core candidate
+ *     pass when norm_bf16 is given, exact fp32 scan when it is NULL) for k + 3 entries, then a, b, c dropped: exact,
+ *     since the top-k outside three ids is a subset of the top-(k+3).
+ *   GLOVE_ANALOGY_MUL (3CosMul, Levy & Goldberg 2014, "Linguistic Regularities in Sparse and Explicit Word
+ *     Representations"): score = ((1+cos(x,b))/2 * (1+cos(x,c))/2) / ((1+cos(x,a))/2 + 1e-3), exact fp32 scan, in a
+ *     fixed operation order (bit-identical from run to run).
+ * Candidates are rows [0, V) of table (V may be smaller than the table: the most frequent words of a frequency-ordered
+ * vocabulary); abc int32 [n][3] device, ids < V (checked by the caller); 1 <= k <= 29 and k + 3 <= V; out_score fp32 and
+ * out_idx int32 [n][k], descending. inv_norm as glove_normalize_rows computes it for the table. */
+enum { GLOVE_ANALOGY_ADD = 0, GLOVE_ANALOGY_MUL = 1 };
+size_t glove_analogy_workspace_bytes(int64_t V, int32_t d, int32_t n_questions, int32_t k, int32_t method);
+int glove_analogy_topk(const float *table, int64_t V, int32_t d, int32_t planes, const void *norm_bf16,
+                       const float *inv_norm, const int32_t *abc, int32_t n_questions, int32_t method, int32_t k,
+                       float *out_score, int32_t *out_idx, void *workspace, size_t workspace_bytes, void *stream);
+/* out[i] = cosine of the rows pairs[2i] and pairs[2i+1] (int32 [n][2] device, ids < V), computed as the top-k computes
+ * its similarities (the first row normalised as the query, the second through inv_norm): bit for bit the similarity the
+ * top-k of the first row reports for the second. */
+int glove_pair_cosine(const float *table, int64_t V, int32_t d, int32_t planes, const float *inv_norm,
+                      const int32_t *pairs, int32_t n_pairs, float *out, void *stream);
+
 /* ---- INGEST: interaction.csv text -> device COO (SURVEY 8 f.1) -----------------------------------------------------
  * Replaces tf.data make_csv_dataset(select_columns=...) [ref src/models/data_utils.py:4-26] and the per-step
  * StaticHashTable(TextFileInitializer(vocab.txt), default_value=0) lookup [ref src/models/model_utils.py:121-127,
