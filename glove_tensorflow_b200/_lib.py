@@ -120,6 +120,14 @@ SIGNATURES = {
                                        c_void, c_void, c_i64, c_void, c_void, c_void, c_void, c_void, c_i64, c_i64,
                                        ctypes.POINTER(c_i64), ctypes.POINTER(c_i64), c_void]),
     "glove_parse_float32": (ctypes.c_int, [ctypes.c_char_p, c_i32, ctypes.POINTER(c_f32)]),
+    "glove_vectors_workspace_bytes": (c_size, [c_i64, c_i64]),
+    "glove_vectors_index": (ctypes.c_int, [c_void, c_i64, c_void, c_size, ctypes.POINTER(c_i64), c_void]),
+    "glove_vectors_parse": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_i64, c_void, c_size, c_void, c_i64, c_i64, c_void,
+                                           c_void, c_i64, ctypes.POINTER(c_i64), ctypes.POINTER(c_i64), c_void]),
+    "glove_vectors_format_size": (ctypes.c_int, [c_void, c_i64, c_i32, c_i64, c_void, c_void, c_size, ctypes.POINTER(c_i64),
+                                                 c_void]),
+    "glove_vectors_format": (ctypes.c_int, [c_void, c_i64, c_i32, c_i64, c_void, c_void, c_void, c_size, c_void, c_i64, c_void]),
+    "glove_format_float32": (ctypes.c_int, [c_f32, ctypes.c_char_p, c_i32, ctypes.POINTER(c_i32)]),
     "glove_tokens_workspace_bytes": (c_size, [c_i64, c_i64]),
     "glove_tokens_scan": (ctypes.c_int, [c_void, c_i64, c_void, c_size, c_void, c_void, c_i64, ctypes.POINTER(c_i64), c_void]),
     "glove_tokens_count": (ctypes.c_int, [c_void, c_i64, c_void, c_i64, c_void, c_size, c_void, c_void, c_void, c_i64,

@@ -192,7 +192,17 @@ class GloveEngine:
             assert e.shape == (self.V, self.d) and b.shape == (self.V,)
             check(lib.glove_pack_plane(_ptr(table), self.V, self.d, self.P, 0, side, _ptr(e), _ptr(b), _stream()), "glove_pack_plane")
         self._write_scalars(g=float(g))
+        self._norm_cache = None       # keyed on the step: a replaced table at the same step must not reuse it
         torch.cuda.synchronize()
+
+    def row_plane(self) -> torch.Tensor:
+        """[V, S] view of the row table of a one-plane (SGD) engine, to write rows in place (columns [0, d) are the
+        embedding, the bias and last_step columns stay as they are); forgets the normalised copy of the top-k."""
+        if self.P != 1 or self.sharded:
+            raise RuntimeError("row_plane is for a one-plane (SGD) engine on one GPU")
+        self._join_side()
+        self._norm_cache = None
+        return self.row_table.view(self.V, self.S)
 
     def _local_rows(self, a):
         """Rows of a global [V, ...] array owned by this rank (owned_ids()), zero-padded to V_rows."""

@@ -4,6 +4,11 @@ SimLex / MEN style ``w1 w2 score`` files), from a checkpoint of a job directory.
 
     python -m glove_tensorflow_b200.evaluate_embeddings --job-dir J [--checkpoint P] [--analogies FILE ...]
         [--similarity FILE ...] [--restrict-vocab N] [--vectors row|sum] [--case-sensitive] [--output-json PATH]
+    python -m glove_tensorflow_b200.evaluate_embeddings --vectors-txt FILE [--dim D] --output-json PATH [...]
+
+``--vectors-txt`` evaluates any word-vectors file in the GloVe text format (Stanford's trainer, the published glove.*
+files, gensim's word2vec text format; see vectors.py), parsed on the GPU; the candidates and ``--restrict-vocab`` follow
+the file's order (published files are in frequency order).
 
 Conventions (Stanford GloVe ``eval/python/evaluate.py``; 3CosMul after Levy & Goldberg 2014): rows are l2-normalised,
 the answer to a : b :: c : ? is the best row outside the ids of a, b and c, ties go to the lower id.  ``--restrict-vocab
@@ -231,7 +236,11 @@ def log_report(report):
 
 def main(argv=None):
     ap = ArgumentParser(description="Word-analogy and word-similarity evaluation of a trained job's embeddings.")
-    ap.add_argument("--job-dir", required=True, help="job directory (params.json, vocab.txt, checkpoints)")
+    src = ap.add_mutually_exclusive_group(required=True)
+    src.add_argument("--job-dir", help="job directory (params.json, vocab.txt, checkpoints)")
+    src.add_argument("--vectors-txt", metavar="FILE", help="word vectors in the GloVe text format (optional word2vec header)")
+    ap.add_argument("--dim", type=int, default=None, metavar="D",
+                    help="with --vectors-txt: the number of values per line (default: from the header or the first line)")
     ap.add_argument("--checkpoint", default=None, help="checkpoint file (default: the latest in the job directory)")
     ap.add_argument("--analogies", nargs="+", action="extend", default=[], metavar="FILE",
                     help="analogy files in questions-words.txt format")
@@ -239,15 +248,28 @@ def main(argv=None):
                     help="word-similarity files: 'w1 w2 score' per line")
     ap.add_argument("--restrict-vocab", type=int, default=None, metavar="N",
                     help="only the first N words of vocab.txt (the most frequent) are looked up and ranked")
-    ap.add_argument("--vectors", choices=("row", "sum"), default="row",
-                    help="row: the row embeddings (PREDICT and export use them); sum: row + column embeddings")
+    ap.add_argument("--vectors", choices=("row", "sum"), default=None,
+                    help="row (default): the row embeddings (PREDICT and export use them); sum: row + column embeddings")
     ap.add_argument("--case-sensitive", action="store_true", help="match words exactly (default: lower() on both sides)")
-    ap.add_argument("--output-json", default=None, help="report path (default: <job-dir>/intrinsic_eval.json)")
+    ap.add_argument("--output-json", default=None,
+                    help="report path (default: <job-dir>/intrinsic_eval.json; required with --vectors-txt)")
     args = ap.parse_args(argv)
     if args.restrict_vocab is not None and args.restrict_vocab < 1:
         ap.error("--restrict-vocab must be at least 1")
-    eng, vocab, ckpt, step = load_engine(args.job_dir, args.checkpoint, args.vectors)
-    report = {"checkpoint": ckpt, "global_step": step, "vectors": args.vectors}
+    if args.vectors_txt is not None:
+        if args.output_json is None:
+            ap.error("--vectors-txt needs --output-json")
+        if args.vectors is not None or args.checkpoint is not None:
+            ap.error("--vectors and --checkpoint apply to --job-dir only")
+        from .vectors import vectors_engine
+        eng, vocab = vectors_engine(args.vectors_txt, args.dim)
+        report = {"vectors_txt": args.vectors_txt, "rows": eng.V, "dim": eng.d}
+    else:
+        if args.dim is not None:
+            ap.error("--dim applies to --vectors-txt only")
+        vectors = args.vectors or "row"
+        eng, vocab, ckpt, step = load_engine(args.job_dir, args.checkpoint, vectors)
+        report = {"checkpoint": ckpt, "global_step": step, "vectors": vectors}
     report.update(evaluate(eng, vocab, args.analogies, args.similarity, args.restrict_vocab, args.case_sensitive))
     log_report(report)
     out = args.output_json or os.path.join(args.job_dir, "intrinsic_eval.json")

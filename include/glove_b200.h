@@ -360,6 +360,44 @@ int glove_csv_parse(const uint8_t *text, int64_t nbytes, int32_t final_chunk, vo
 /* Host entry to the decimal -> float32 routine the parse kernel uses (one field, no blanks); for tests and tools. */
 int glove_parse_float32(const char *text, int32_t n, float *out);
 
+/* ---- WORD VECTORS: the GloVe text format <-> device float32 rows (glove_vectors.cu) -------------------------------
+ * Format (DESIGN.md 3): one vector per line, "word v_1 ... v_d"; fields separated by runs of ASCII space / tab; trailing
+ * blanks and a '\r' before the '\n' ignored; blank lines skipped; the LAST d fields are the numbers and the word is
+ * everything before them with the separating blanks trimmed (words may contain spaces or look like numbers).  Numbers are
+ * rounded once, decimal text -> float32 (glove_parse_float32); nan / inf and malformed numbers fail the call.  The optional
+ * word2vec header "V d" and the choice of d (2 <= d <= 510) are the caller's business (they need the first line only).
+ * Import: the caller uploads the file chunk by chunk (text: device, 16-byte aligned, every chunk starts at a line start),
+ * glove_vectors_index counts its '\n', glove_vectors_parse (same text, nbytes and workspace) parses it.  Export: rows are
+ * printed with the shortest decimal that parses back to the same float32 (glove_format_float32). */
+/* n_lines = the count glove_vectors_index returned (0 for the index call itself), or the number of rows to format with
+ * nbytes = 0. */
+size_t glove_vectors_workspace_bytes(int64_t nbytes, int64_t n_lines);
+/* Number of '\n' in the chunk -> *n_lines_host.  Synchronises the stream. */
+int glove_vectors_index(const uint8_t *text, int64_t nbytes, void *workspace, size_t workspace_bytes, int64_t *n_lines_host,
+                        void *stream);
+/* Parses the non-blank lines of the chunk in order: row r of the chunk goes to out + r * ld (ld >= d floats, so that a
+ * packed one-plane table, ld = glove_table_stride(d), is filled in place), its word to text[word_start[r] ..
+ * + word_len[r]).  A row past row_capacity fails the call (a header's count).  final_chunk: an unterminated last line is
+ * parsed; otherwise its bytes are left to the next chunk (*consumed_host = bytes of this chunk that were parsed).
+ * first_line = 1-based file line of the chunk's first line (lines of padding in front count), for the error message,
+ * which names the lowest offending line.
+ * Synchronises. */
+int glove_vectors_parse(const uint8_t *text, int64_t nbytes, int32_t final_chunk, int32_t d, int64_t n_lines,
+                        void *workspace, size_t workspace_bytes, float *out, int64_t ld, int64_t row_capacity,
+                        int64_t *word_start, int32_t *word_len, int64_t first_line, int64_t *n_rows_host,
+                        int64_t *consumed_host, void *stream);
+/* Export of n rows (rows: device fp32, leading dimension ld) with their words (words[word_off[r] .. word_off[r+1]), word_off
+ * device int64 [n + 1]) as n lines "word v_1 ... v_d\n".  format_size computes the line offsets in the workspace
+ * (glove_vectors_workspace_bytes(0, n)) and the text size (synchronises); format, on the same arguments and workspace,
+ * writes the text (capacity >= that size; asynchronous after one read of the size). */
+int glove_vectors_format_size(const float *rows, int64_t ld, int32_t d, int64_t n, const int64_t *word_off, void *workspace,
+                              size_t workspace_bytes, int64_t *text_bytes_host, void *stream);
+int glove_vectors_format(const float *rows, int64_t ld, int32_t d, int64_t n, const uint8_t *words, const int64_t *word_off,
+                         void *workspace, size_t workspace_bytes, uint8_t *text, int64_t capacity, void *stream);
+/* Host entry to the float32 -> shortest decimal routine the export kernel uses: out (capacity >= 16) receives *length
+ * bytes, no terminating NUL.  For tests and tools. */
+int glove_format_float32(float value, char *out, int32_t capacity, int32_t *length);
+
 /* ---- TOKENS: corpus text -> token stream, the front half of the preprocessor (SURVEY 8 f.4) ------------------------
  * text8.split() [ref src/data/text8.py:47], Counter(text_tokens) [ref :62], token2id.get(token, 0) [ref :85-86].
  * Tokens are maximal runs of non-whitespace bytes (ASCII whitespace; the UTF-8 encodings of the other separators that
