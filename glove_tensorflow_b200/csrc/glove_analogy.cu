@@ -166,15 +166,11 @@ __global__ void __launch_bounds__(256) pair_cosine_kernel(const float *__restric
     load_unit_row(table, S, P, d, pairs[2 * i], qn, S, lane);
     __syncwarp();
     const int32_t v = pairs[2 * i + 1];
-    const int S4 = S >> 2;
     const float *row = table + (int64_t)v * P * S;
     float4 x[NV];
 #pragma unroll
-    for (int r = 0; r < NV; ++r) {
-        const int f = lane + 32 * r;
-        x[r] = f < S4 ? ld4(row + 4 * f) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    const float s = cos_dot<NV>(qn, x, inv_norm[v], lane, S4);
+    for (int r = 0; r < NV; ++r) x[r] = ld4_emb(row, lane + 32 * r, d);
+    const float s = cos_dot<NV>(qn, x, inv_norm[v], lane, S >> 2);
     if (lane == 0) out[i] = s;
 }
 

@@ -69,10 +69,7 @@ __global__ void __launch_bounds__(256) scan_fp32_kernel(const float *__restrict_
         const float *row = table + v * P * S;
         const float rn = inv_norm[v];
 #pragma unroll
-        for (int r = 0; r < NV; ++r) {
-            const int f = lane + 32 * r;
-            x[r] = f < S4 ? ld4(row + 4 * f) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
+        for (int r = 0; r < NV; ++r) x[r] = ld4_emb(row, lane + 32 * r, d);
 #pragma unroll
         for (int t = 0; t < kScanQT; ++t) {
             const float sim = cos_dot<NV>(qn + t * S, x, rn, lane, S4);

@@ -18,8 +18,22 @@ __device__ __forceinline__ float row_inv_norm(const float *__restrict__ row, int
     return 1.0f / sqrtf(fmaxf(ss, 1e-12f));
 }
 
-// sim = sum_c qn[c] * (x[c] * rn): qn = normalised query (zero outside columns < d, so the bias / last_step columns of the
-// packed row drop out), x = packed table row held as NV float4 per lane, rn = its inverse norm.
+// float4 number f of a packed row with the columns >= d (bias, last_step, padding) read as zero: nothing stored there, not
+// even a non-finite bias, reaches a similarity (0 * inf is NaN).  Bit-identical to the plain load for finite values.
+__device__ __forceinline__ float4 ld4_emb(const float *__restrict__ row, int f, int d) {
+    const int c = 4 * f;
+    float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (c < d) {
+        x = ld4(row + c);
+        if (c + 1 >= d) x.y = 0.0f;
+        if (c + 2 >= d) x.z = 0.0f;
+        if (c + 3 >= d) x.w = 0.0f;
+    }
+    return x;
+}
+
+// sim = sum_c qn[c] * (x[c] * rn): qn = normalised query (zero outside columns < d), x = packed table row held as NV
+// float4 per lane (ld4_emb: zero outside columns < d), rn = its inverse norm.
 template <int NV>
 __device__ __forceinline__ float cos_dot(const float *__restrict__ qn, const float4 (&x)[NV], float rn, int lane, int S4) {
     float p = 0.0f;

@@ -307,10 +307,7 @@ __global__ void __launch_bounds__(256) rescore_kernel(const float *__restrict__ 
         float4 x[NV];
         const float *row = table + (int64_t)v * P * S;
 #pragma unroll
-        for (int r = 0; r < NV; ++r) {
-            const int f = lane + 32 * r;
-            x[r] = f < S4 ? ld4(row + 4 * f) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
+        for (int r = 0; r < NV; ++r) x[r] = ld4_emb(row, lane + 32 * r, d);
         top.insert(cos_dot<NV>(qn, x, inv_norm[v], lane, S4), v, lane, k);
     }
     if (lane < k) {

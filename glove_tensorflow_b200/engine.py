@@ -223,6 +223,8 @@ class GloveEngine:
     def set_plane(self, side: str, plane: int, emb: torch.Tensor, bias: torch.Tensor):
         """Write optimizer slot plane ``plane`` (1 = Adam m / Adagrad acc, 2 = Adam v) of ``side`` in {'row','col'}."""
         self._join_side()
+        if plane == 0 and side == "row":
+            self._norm_cache = None   # the embedding plane itself: the normalised copy of the top-k is stale
         table = self.row_table if side == "row" else self.col_table
         check(lib.glove_pack_plane(_ptr(table), self.V, self.d, self.P, plane, 0 if side == "row" else 1,
                                    _ptr(emb.contiguous()), _ptr(bias.contiguous()), _stream()), "glove_pack_plane")
@@ -258,6 +260,7 @@ class GloveEngine:
                 b2[: ids.numel()] = b[ids]
                 e, b = e2, b2
             check(lib.glove_pack_plane(_ptr(table), self.V, self.d, self.P, 0, side, _ptr(e), _ptr(b), _stream()), "glove_pack_plane")
+        self._norm_cache = None       # as in load_state: a new table at the same step must not be ranked with old norms
         torch.cuda.synchronize()
 
     def _unpack(self, table, plane):

@@ -127,3 +127,19 @@ def planted_analogies(n_groups, D, seed=0):
         vocab += ["w%d" % g, "W%d_off" % g]
         rows += [np.concatenate([base, [1.0, 0.0]]), np.concatenate([base, [0.0, 1.0]])]
     return vocab, np.array(rows, np.float32)
+
+
+MUL_QT, MUL_TV, NUM_SMS = 8, 256, 148      # kMulQT, kMulTV (glove_analogy.cu), kNumSMs (glove_common.cuh)
+
+
+def mul_plan(V, n):
+    """(question tiles, table slices, rows per slice) of the 3CosMul scan for n questions over V rows -- mul_plan of
+    glove_analogy.cu: at least two CTAs per SM, at most 64 slices and no more slices than 256-row tiles.  Slice s holds
+    rows [s * rows_per_slice, min((s + 1) * rows_per_slice, V)) and sweeps them in 256-row tiles from its first row, one
+    32-row warp list per tile section; the tests plant exact ties on these edges."""
+    q_tiles = (n + MUL_QT - 1) // MUL_QT
+    slices = min((2 * NUM_SMS + q_tiles - 1) // q_tiles, 64)
+    if slices * MUL_TV > V:
+        slices = (V + MUL_TV - 1) // MUL_TV
+    slices = max(slices, 1)
+    return q_tiles, slices, (V + slices - 1) // slices

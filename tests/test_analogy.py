@@ -162,6 +162,29 @@ def test_oracle_normalisation_floor():
     assert np.all(n[0] == 0) and abs(n[1][0] - 1e-8 / 1e-6) < 1e-18
 
 
+def test_mul_plan_restates_the_kernel():
+    """The 3CosMul slicing the edge tests plant ties against: the constants are the kernel's, every row is in exactly one
+    non-empty slice, and the extremes fall where the GPU tests expect them."""
+    import os
+    import re
+    csrc = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "glove_tensorflow_b200", "csrc")
+    src = open(os.path.join(csrc, "glove_analogy.cu")).read()
+    assert int(re.search(r"constexpr int kMulQT = (\d+);", src).group(1)) == ao.MUL_QT
+    assert int(re.search(r"constexpr int kMulTV = (\d+);", src).group(1)) == ao.MUL_TV
+    assert "if (slices > 64) slices = 64;" in src and "(2 * kNumSMs + p.q_tiles - 1) / p.q_tiles" in src
+    common = open(os.path.join(csrc, "glove_common.cuh")).read()
+    assert int(re.search(r"constexpr int kNumSMs = (\d+);", common).group(1)) == ao.NUM_SMS
+    for V in (4, 31, 255, 256, 257, 1023, 1024, 5249, 16384, 16411, 20000, 400000):
+        for n in (1, 7, 8, 9, 300, 2368, 2369, 2500):
+            q_tiles, slices, rps = ao.mul_plan(V, n)
+            assert q_tiles * ao.MUL_QT >= n > (q_tiles - 1) * ao.MUL_QT
+            assert 1 <= slices <= 64 and (slices - 1) * rps < V <= slices * rps
+            assert slices <= (V + ao.MUL_TV - 1) // ao.MUL_TV     # no more slices than 256-row tiles
+    assert ao.mul_plan(16384, 1) == (1, 64, 256) and ao.mul_plan(20000, 9) == (2, 64, 313)
+    assert ao.mul_plan(20000, 2368)[1] == 1 and ao.mul_plan(5249, 2369)[1] == 1 and ao.mul_plan(5249, 2360)[1] == 2
+    assert ao.mul_plan(255, 1) == (1, 1, 255) and ao.mul_plan(257, 1) == (1, 2, 129)
+
+
 def test_correlations_match_scipy():
     rng = np.random.default_rng(3)
     for n in (2, 5, 40, 300):
