@@ -141,6 +141,23 @@ SIGNATURES = {
     "glove_cooc_finish": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, c_i32, c_i64, c_void, c_i64, ctypes.c_uint64, c_void,
                                          c_size, c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64,
                                          ctypes.POINTER(c_i64), c_void]),
+    "glove_cooc_route_workspace_bytes": (c_size, [c_i64, c_i32]),
+    "glove_cooc_route": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, ctypes.c_uint64, c_i32, c_void, c_size, c_void, c_void,
+                                        c_i64, c_void, c_void]),
+    "glove_cooc_finish_sorted": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, c_i32, c_i64, c_void, c_i64, ctypes.c_uint64,
+                                                c_void, c_size, c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64,
+                                                ctypes.POINTER(c_i64), c_void]),
+    "glove_vocab_merge_workspace_bytes": (c_size, [c_i64, c_i64]),
+    "glove_vocab_merge": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_void, c_i64, c_void, c_void, c_void, c_void, c_void,
+                                         c_i64, c_void, c_i64, c_i64, c_void, c_size, c_void, c_void, c_void, c_void, c_void,
+                                         c_i64, ctypes.POINTER(c_i64), ctypes.POINTER(c_i64), c_void]),
+    "glove_cooc_csv_workspace_bytes": (c_size, [c_i64]),
+    "glove_cooc_csv_size": (ctypes.c_int, [c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64, c_void, c_void,
+                                           c_size, ctypes.POINTER(c_i64), c_void]),
+    "glove_cooc_csv_format": (ctypes.c_int, [c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64, c_void, c_void,
+                                             c_void, c_size, c_void, c_i64, c_void]),
+    "glove_format_float64": (ctypes.c_int, [ctypes.c_double, ctypes.c_char_p, c_i32, ctypes.POINTER(c_i32)]),
+    "glove_format_float64_device": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_void]),
     "glove_host_staging_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_plan_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_pipe_create": (ctypes.c_int, [ctypes.POINTER(c_void)]),

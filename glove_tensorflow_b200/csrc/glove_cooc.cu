@@ -21,6 +21,8 @@
 
 namespace glove {
 
+constexpr int kCoocMaxPartBits = 12;   // glove_cooc_route: at most 4096 partitions
+
 struct Agg { long long count, numer; };
 struct AggSum {
     __host__ __device__ __forceinline__ Agg operator()(const Agg &a, const Agg &b) const {
@@ -169,8 +171,95 @@ __global__ void __launch_bounds__(256) columns_kernel(const uint64_t *__restrict
     glove_value[i] = log(v);
 }
 
+// partition of a directed key: the top part_bits bits of its order hash, so that the partitions taken in ascending order
+// and each sorted by the full hash give the single-table record order
+__device__ __forceinline__ uint32_t part_of(uint64_t key, uint64_t salt, int part_bits) {
+    return part_bits ? (uint32_t)(mix64(key + salt * 0x9e3779b97f4a7c15ull) >> (64 - part_bits)) : 0u;
+}
+__device__ __forceinline__ uint64_t directed_key(const uint64_t *keys, int64_t n, int64_t t, int vbits) {
+    const uint64_t k = keys[t < n ? t : t - n], mask = (1ull << vbits) - 1;
+    return t < n ? k : ((k & mask) << vbits) | (k >> vbits);
+}
+// t < n: entry t as (a, b); t >= n: entry t - n as (b, a)
+__global__ void __launch_bounds__(256) route_parts_kernel(const uint64_t *__restrict__ keys, int64_t n, int vbits, uint64_t salt,
+                                                          int part_bits, uint32_t *part, uint32_t *idx) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= 2 * n) return;
+    part[t] = part_of(directed_key(keys, n, t, vbits), salt, part_bits);
+    idx[t] = (uint32_t)t;
+}
+__global__ void __launch_bounds__(256) route_scatter_kernel(const uint64_t *__restrict__ keys, const Agg *__restrict__ agg,
+                                                            int64_t n, int vbits, const uint32_t *__restrict__ order,
+                                                            uint64_t *out_keys, Agg *out_agg) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 2 * n) return;
+    const int64_t t = order[i];
+    out_keys[i] = directed_key(keys, n, t, vbits);
+    out_agg[i] = agg[t < n ? t : t - n];
+}
+
+struct RouteWs {
+    uint32_t *part[2], *idx[2];
+    int *hist;
+    void *cub_temp;
+    size_t cub_bytes, bytes;
+};
+static RouteWs route_ws_view(void *base, int64_t n2, int part_bits) {
+    RouteWs w;
+    char *p = (char *)base;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char *r = p ? p + off : nullptr; off += align_up(bytes); return r; };
+    for (int i = 0; i < 2; ++i) w.part[i] = (uint32_t *)take(4 * n2);
+    for (int i = 0; i < 2; ++i) w.idx[i] = (uint32_t *)take(4 * n2);
+    w.hist = (int *)take(sizeof(int) << part_bits);
+    size_t a = 0, b = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, a, (uint32_t *)nullptr, (uint32_t *)nullptr, (uint32_t *)nullptr, (uint32_t *)nullptr,
+                                    (int)n2);
+    cub::DeviceHistogram::HistogramEven(nullptr, b, (uint32_t *)nullptr, (int *)nullptr, (1 << part_bits) + 1, 0u,
+                                        (uint32_t)(1 << part_bits), (int)n2);
+    w.cub_bytes = a > b ? a : b;
+    w.cub_temp = take(w.cub_bytes);
+    w.bytes = off;
+    return w;
+}
+
 static int read_count(const long long *dev, long long *host, cudaStream_t stream) {
     GLOVE_CHECK_CUDA(cudaMemcpyAsync(host, dev, sizeof(long long), cudaMemcpyDeviceToHost, stream));
+    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    return GLOVE_OK;
+}
+
+// records of a summed symmetric table (keys sorted ascending, unique): count >= count_min, in the keyed-hash order
+// (a stable sort of the ascending keys by mix64(key + salt phi): equal hashes keep key order), with the GloVe columns
+static int finish_records(const char *who, const uint64_t *keys, const Agg *agg, long long m, const CoocWs &w, int vbits,
+                          int32_t context, int64_t count_min, const int64_t *vocab_count, int64_t total_tokens,
+                          uint64_t order_key, int32_t *row, int32_t *col, int64_t *count, double *value, double *neg_weight,
+                          double *glove_weight, double *glove_value, int64_t capacity, int64_t *n_out_host,
+                          cudaStream_t stream) {
+    // count >= count_minimum
+    flag_min_count_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>(agg, m, count_min, w.flags, w.idx[0]);
+    GLOVE_CHECK_LAUNCH();
+    size_t tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceSelect::Flagged(w.cub_temp, tb, w.idx[0], w.flags, w.idx[1], w.count_out, (int)m, stream));
+    long long n_out = 0;
+    if (int rc = read_count(w.count_out, &n_out, stream)) return rc;
+    *n_out_host = n_out;
+    if (n_out > capacity)
+        return set_error(GLOVE_EINVAL, "%s: %lld records > capacity %lld", who, n_out, (long long)capacity);
+    if (n_out == 0) return GLOVE_OK;
+    GLOVE_REQUIRE(row && col && count && value && neg_weight && glove_weight && glove_value, "%s: null output", who);
+    // keyed-hash record order
+    const unsigned go = (unsigned)((n_out + 255) / 256);
+    order_keys_kernel<<<go, 256, 0, stream>>>(keys, w.idx[1], n_out, order_key, w.keys[2]);
+    GLOVE_CHECK_LAUNCH();
+    tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.keys[2], w.keys[3], w.idx[1], w.idx[0], (int)n_out, 0, 64,
+                                                     stream));
+    const long long unit = lcm_upto(context);
+    columns_kernel<<<go, 256, 0, stream>>>(keys, agg, w.idx[0], n_out, vbits, 1.0 / (double)unit, unit,
+                                           (const long long *)vocab_count, (double)total_tokens, row, col,
+                                           (long long *)count, value, neg_weight, glove_weight, glove_value);
+    GLOVE_CHECK_LAUNCH();
     GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
     return GLOVE_OK;
 }
@@ -293,32 +382,73 @@ int glove_cooc_finish(const uint64_t *keys, const int64_t *agg, int64_t n, int32
                                                     (int)n2, stream));
     long long m = 0;
     if (int rc = read_count(w.count_out, &m, stream)) return rc;
-    // count >= count_minimum
-    flag_min_count_kernel<<<(unsigned)((m + 255) / 256), 256, 0, stream>>>(w.agg2, m, count_min, w.flags, w.idx[0]);
+    return finish_records("glove_cooc_finish", w.keys[0], w.agg2, m, w, vbits, context, count_min, vocab_count, total_tokens,
+                          order_key, row, col, count, value, neg_weight, glove_weight, glove_value, capacity, n_out_host,
+                          stream);
+}
+
+size_t glove_cooc_route_workspace_bytes(int64_t n, int32_t part_bits) {
+    return route_ws_view(nullptr, 2 * (n < 1 ? 1 : n), part_bits < 0 ? 0 : part_bits > kCoocMaxPartBits ? kCoocMaxPartBits : part_bits).bytes;
+}
+
+int glove_cooc_route(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, uint64_t order_key, int32_t part_bits,
+                     void *workspace, size_t workspace_bytes, uint64_t *out_keys, int64_t *out_agg, int64_t capacity,
+                     int64_t *part_count_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(keys && agg && workspace && out_keys && out_agg && part_count_host, "glove_cooc_route: null pointer");
+    GLOVE_REQUIRE(n > 0 && V > 1 && part_bits >= 0 && part_bits <= kCoocMaxPartBits,
+                  "glove_cooc_route: bad sizes (part_bits must be 0..%d)", kCoocMaxPartBits);
+    GLOVE_REQUIRE(2 * n < (1ll << 31), "glove_cooc_route: more than 2^30 entries");
+    GLOVE_REQUIRE(capacity >= 2 * n, "glove_cooc_route: capacity %lld < 2n = %lld", (long long)capacity, (long long)(2 * n));
+    const int vbits = vbits_of((int64_t)V + 1);
+    const int64_t n2 = 2 * n;
+    const RouteWs w = route_ws_view(workspace, n2, part_bits);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "glove_cooc_route: workspace %zu < required %zu", workspace_bytes, w.bytes);
+    const unsigned g = (unsigned)((n2 + 255) / 256);
+    route_parts_kernel<<<g, 256, 0, stream>>>(keys, n, vbits, order_key, part_bits, w.part[0], w.idx[0]);
     GLOVE_CHECK_LAUNCH();
-    tb = w.cub_bytes;
-    GLOVE_CHECK_CUDA(cub::DeviceSelect::Flagged(w.cub_temp, tb, w.idx[0], w.flags, w.idx[1], w.count_out, (int)m, stream));
-    long long n_out = 0;
-    if (int rc = read_count(w.count_out, &n_out, stream)) return rc;
-    *n_out_host = n_out;
-    if (n_out > capacity)
-        return set_error(GLOVE_EINVAL, "glove_cooc_finish: %lld records > capacity %lld", n_out, (long long)capacity);
-    if (n_out == 0) return GLOVE_OK;
-    GLOVE_REQUIRE(row && col && count && value && neg_weight && glove_weight && glove_value, "glove_cooc_finish: null output");
-    // keyed-hash record order
-    const unsigned go = (unsigned)((n_out + 255) / 256);
-    order_keys_kernel<<<go, 256, 0, stream>>>(w.keys[0], w.idx[1], n_out, order_key, w.keys[2]);
+    const uint32_t *order = w.idx[0];
+    const int P = 1 << part_bits;
+    if (part_bits) {
+        size_t tb = w.cub_bytes;
+        GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.part[0], w.part[1], w.idx[0], w.idx[1], (int)n2, 0,
+                                                         part_bits, stream));
+        tb = w.cub_bytes;
+        GLOVE_CHECK_CUDA(cub::DeviceHistogram::HistogramEven(w.cub_temp, tb, w.part[1], w.hist, P + 1, 0u, (uint32_t)P, (int)n2,
+                                                             stream));
+        order = w.idx[1];
+    }
+    route_scatter_kernel<<<g, 256, 0, stream>>>(keys, (const Agg *)agg, n, vbits, order, out_keys, (Agg *)out_agg);
     GLOVE_CHECK_LAUNCH();
-    tb = w.cub_bytes;
-    GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.keys[2], w.keys[3], w.idx[1], w.idx[0], (int)n_out, 0, 64,
-                                                     stream));
-    const long long unit = lcm_upto(context);
-    columns_kernel<<<go, 256, 0, stream>>>(w.keys[0], w.agg2, w.idx[0], n_out, vbits, 1.0 / (double)unit, unit,
-                                           (const long long *)vocab_count, (double)total_tokens, row, col,
-                                           (long long *)count, value, neg_weight, glove_weight, glove_value);
-    GLOVE_CHECK_LAUNCH();
-    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    if (part_bits) {
+        int hist[1 << kCoocMaxPartBits];
+        GLOVE_CHECK_CUDA(cudaMemcpyAsync(hist, w.hist, sizeof(int) * P, cudaMemcpyDeviceToHost, stream));
+        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+        for (int p = 0; p < P; ++p) part_count_host[p] = hist[p];
+    } else {
+        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+        part_count_host[0] = n2;
+    }
     return GLOVE_OK;
+}
+
+int glove_cooc_finish_sorted(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t context, int64_t count_min,
+                             const int64_t *vocab_count, int64_t total_tokens, uint64_t order_key, void *workspace,
+                             size_t workspace_bytes, int32_t *row, int32_t *col, int64_t *count, double *value,
+                             double *neg_weight, double *glove_weight, double *glove_value, int64_t capacity,
+                             int64_t *n_out_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(keys && agg && vocab_count && workspace && n_out_host && n > 0, "glove_cooc_finish_sorted: bad arguments");
+    GLOVE_REQUIRE(context >= 1 && context <= 8 && total_tokens > 0 && V > 1, "glove_cooc_finish_sorted: bad sizes");
+    GLOVE_REQUIRE(n < (1ll << 31), "glove_cooc_finish_sorted: more than 2^31 entries");
+    const int vbits = vbits_of((int64_t)V + 1);
+    const CoocWs w = cooc_ws_view(workspace, n);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "glove_cooc_finish_sorted: workspace %zu < required %zu", workspace_bytes, w.bytes);
+    return finish_records("glove_cooc_finish_sorted", keys, (const Agg *)agg, n, w, vbits, context, count_min, vocab_count,
+                          total_tokens, order_key, row, col, count, value, neg_weight, glove_weight, glove_value, capacity,
+                          n_out_host, stream);
 }
 
 }  // extern "C"

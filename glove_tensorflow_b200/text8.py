@@ -264,7 +264,8 @@ def main(argv=None):
     args = ap.parse_args(argv)
     logger.info("call: %s.", " ".join(sys.argv))
     download_data(args.url, args.dest)
-    save_data(process_data(load_data(args.dest), args.vocab_size, args.coverage, args.context_size, args.device), args.dest)
+    from .corpus import preprocess     # the streamed preprocessor: same files as save_data(process_data(...))
+    preprocess(os.path.join(args.dest, "text8"), args.dest, args.vocab_size, args.coverage, args.context_size, args.device)
 
 
 if __name__ == "__main__":

@@ -444,6 +444,54 @@ int glove_cooc_finish(const uint64_t *keys, const int64_t *agg, int64_t n, int32
                       size_t workspace_bytes, int32_t *row, int32_t *col, int64_t *count, double *value, double *neg_weight,
                       double *glove_weight, double *glove_value, int64_t capacity, int64_t *n_out_host, void *stream);
 
+/* Streamed preprocessing (glove_tensorflow_b200/corpus.py): the co-occurrence table split into 2^part_bits partitions by
+ * the top bits of the record-order hash, each merged and finished on its own; taken in ascending order the partitions'
+ * records are the record order of glove_cooc_finish.  glove_cooc_route writes both orientations of every entry of a
+ * right-context table (keys, agg as from glove_cooc_chunk) grouped by partition: partition p is the next
+ * part_count_host[p] entries of out_keys / out_agg (capacity >= 2n).  part_bits 0..12.  Synchronises. */
+size_t glove_cooc_route_workspace_bytes(int64_t n, int32_t part_bits);
+int glove_cooc_route(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, uint64_t order_key, int32_t part_bits,
+                     void *workspace, size_t workspace_bytes, uint64_t *out_keys, int64_t *out_agg, int64_t capacity,
+                     int64_t *part_count_host, void *stream);
+/* glove_cooc_finish for a table that is already symmetric (one partition merged from routed entries): no transpose.
+ * Workspace: glove_cooc_workspace_bytes(n). */
+int glove_cooc_finish_sorted(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t context, int64_t count_min,
+                             const int64_t *vocab_count, int64_t total_tokens, uint64_t order_key, void *workspace,
+                             size_t workspace_bytes, int32_t *row, int32_t *col, int64_t *count, double *value,
+                             double *neg_weight, double *glove_weight, double *glove_value, int64_t capacity,
+                             int64_t *n_out_host, void *stream);
+/* Pass 1 of the streamed preprocessor: merges the n_chunk distinct tokens of one text chunk (first / first_len / count
+ * as from glove_tokens_count; origin = byte offset of text[0] in the corpus) into the global table of distinct tokens
+ * (g_*, n_global entries sorted by token hash; g_first = corpus byte offset of the first occurrence, g_off / g_len = the
+ * token bytes in pool).  The merged table goes to o_* (capacity >= n_global + n_chunk suffices), new tokens append their
+ * bytes to pool[pool_used ..]; *pool_used_host receives the new fill.  Equal hashes of different tokens fail with
+ * GLOVE_EUNSUPPORTED.  Synchronises. */
+size_t glove_vocab_merge_workspace_bytes(int64_t n_global, int64_t n_chunk);
+int glove_vocab_merge(const uint8_t *text, int64_t origin, const int64_t *first, const int32_t *first_len, const int64_t *count,
+                      int64_t n_chunk, const uint64_t *g_hash, const int64_t *g_count, const int64_t *g_first,
+                      const int64_t *g_off, const int32_t *g_len, int64_t n_global, uint8_t *pool, int64_t pool_used,
+                      int64_t pool_capacity, void *workspace, size_t workspace_bytes, uint64_t *o_hash, int64_t *o_count,
+                      int64_t *o_first, int64_t *o_off, int32_t *o_len, int64_t capacity, int64_t *n_out_host,
+                      int64_t *pool_used_host, void *stream);
+/* interaction.csv lines of n finished records (the columns of glove_cooc_finish) in the reference's column order:
+ * row_token_id,col_token_id,count,value,row_token,col_token,neg_weight,glove_weight,glove_value.  Token t is
+ * token_bytes[token_off[t] .. token_off[t+1]), already quoted as the csv needs; float64 values print as repr(float).
+ * glove_cooc_csv_size measures (synchronises), glove_cooc_csv_format (same columns and workspace) writes (asynchronous). */
+size_t glove_cooc_csv_workspace_bytes(int64_t n_records);
+int glove_cooc_csv_size(const int32_t *row, const int32_t *col, const int64_t *count, const double *value,
+                        const double *neg_weight, const double *glove_weight, const double *glove_value, int64_t n,
+                        const int64_t *token_off, void *workspace, size_t workspace_bytes, int64_t *text_bytes_host,
+                        void *stream);
+int glove_cooc_csv_format(const int32_t *row, const int32_t *col, const int64_t *count, const double *value,
+                          const double *neg_weight, const double *glove_weight, const double *glove_value, int64_t n,
+                          const uint8_t *token_bytes, const int64_t *token_off, void *workspace, size_t workspace_bytes,
+                          uint8_t *text, int64_t capacity, void *stream);
+/* Host entry to the float64 -> repr(float) routine the csv kernel uses: out (capacity >= 24) receives *length bytes, no
+ * terminating NUL.  glove_format_float64_device runs the device build on n bit patterns (device memory): slot i of out
+ * (24 bytes each) receives len[i] bytes.  Asynchronous.  For tests and tools. */
+int glove_format_float64(double value, char *out, int32_t capacity, int32_t *length);
+int glove_format_float64_device(const uint64_t *bits, int64_t n, char *out, int32_t *len, void *stream);
+
 /* ---- HOST-buffer boundary (end to end): what a non-torch caller of the reference's training path would bind ----- */
 /* Runs K TRAIN steps (K a multiple of args->plan_K, at most 4096) on K*B explicit triples held in HOST memory (pinned
  * recommended) and copies the K losses back to host_losses.  Internally a pipeline over the chunks of plan_K steps:
