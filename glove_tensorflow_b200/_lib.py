@@ -43,6 +43,7 @@ class CsvSchema(ctypes.Structure):
 
 
 CSV_TOKEN, CSV_INT, CSV_FLOAT = 0, 1, 2
+CREC_BAD_WORD1, CREC_BAD_WORD2, CREC_BAD_VALUE = 0, 1, 2   # kinds of glove_cooc_bin_parse's error word
 
 # name -> (restype, argtypes); every symbol include/glove_b200.h declares
 SIGNATURES = {
@@ -158,6 +159,9 @@ SIGNATURES = {
                                              c_void, c_size, c_void, c_i64, c_void]),
     "glove_format_float64": (ctypes.c_int, [ctypes.c_double, ctypes.c_char_p, c_i32, ctypes.POINTER(c_i32)]),
     "glove_format_float64_device": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_void]),
+    "glove_cooc_bin_parse": (ctypes.c_int, [c_void, c_i64, c_i64, c_i64, ctypes.c_double, ctypes.c_double, c_void, c_void,
+                                            c_void, c_void, c_void, c_void]),
+    "glove_cooc_bin_format": (ctypes.c_int, [c_void, c_void, c_void, c_i64, c_void, c_void]),
     "glove_host_staging_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_plan_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_pipe_create": (ctypes.c_int, [ctypes.POINTER(c_void)]),

@@ -1,7 +1,8 @@
 """CLI + job-dir bookkeeping of the trainer: same 19 flags, names, types and defaults as the reference's
 src/models/config_utils.py:76-180, same derived ``input_fn_args`` / ``dataset_args`` / ``serving_input_fn_args`` (:20-45),
 same ``params.json`` (indent 2, :48-52) and vocab copy into the job dir (:55-73).  Flags that only exist here
-(--adam-mode, --reg-scale, --plan-steps, --seed, --device) default to the reference's behaviour."""
+(--adam-mode, --reg-scale, --plan-steps, --seed, --device, --train-cooc, --x-max, --alpha) default to the reference's
+behaviour.  A --vocab-txt of Stanford GloVe's ``word count`` lines is copied into the job dir as one token per line."""
 import json
 import logging
 import os
@@ -14,6 +15,7 @@ from .config import (
     BATCH_SIZE, COL_NAME, EMBEDDING_SIZE, JOB_DIR, L2_REG, LEARNING_RATE, NEG_FACTOR, NEG_NAME, OPTIMIZER, POS_NAME,
     ROW_NAME, STEPS_PER_EPOCH, TARGET_NAME, TOP_K, TRAIN_CSV, TRAIN_STEPS, VOCAB_TXT, WEIGHT_NAME,
 )
+from .data_utils import read_stanford_vocab
 
 logger = logging.getLogger(__name__)
 
@@ -50,7 +52,13 @@ def init_params(params):
         params["job_dir"] = "{job_dir}-{datetime:%Y%m%d-%H%M%S}".format(job_dir=params["job_dir"], datetime=datetime.now())
     os.makedirs(params["job_dir"], exist_ok=True)
     output_vocab_txt = os.path.join(params["job_dir"], os.path.basename(params["vocab_txt"]))
-    if os.path.abspath(params["vocab_txt"]) != os.path.abspath(output_vocab_txt):
+    tokens, counts = read_stanford_vocab(params["vocab_txt"])
+    if counts is not None:
+        # Stanford's `word count` lines: the job-dir copy is one token per line, the vocab.txt every other tool reads
+        with open(output_vocab_txt + ".tmp", "w", encoding="utf8") as f:
+            f.write("\n".join(tokens))
+        os.replace(output_vocab_txt + ".tmp", output_vocab_txt)
+    elif os.path.abspath(params["vocab_txt"]) != os.path.abspath(output_vocab_txt):
         shutil.copyfile(params["vocab_txt"], output_vocab_txt)
     params["vocab_txt"] = output_vocab_txt
     params.update(get_function_args(params))
@@ -90,6 +98,13 @@ def build_parser():
     p.add_argument("--plan-steps", type=int, default=16, help="batches planned per prepare call (default: %(default)s)")
     p.add_argument("--seed", type=int, default=0, help="seed of the table initialiser and the epoch shuffle")
     p.add_argument("--device", default="cuda:0")
+    # --- Stanford GloVe co-occurrence input (glove head only) ---
+    p.add_argument("--train-cooc", default=None,
+                   help="Stanford GloVe cooccurrence.bin / cooccurrence.shuf.bin to train from instead of --train-csv; ids "
+                        "are 1-based lines of --vocab-txt (default: %(default)s)")
+    p.add_argument("--x-max", type=float, default=100.0,
+                   help="with --train-cooc: weight cutoff of glove.c, weight = min(1, (X / x_max)^alpha) (default: %(default)s)")
+    p.add_argument("--alpha", type=float, default=0.75, help="with --train-cooc: weight exponent (default: %(default)s)")
     return p
 
 

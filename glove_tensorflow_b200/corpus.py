@@ -14,10 +14,12 @@ whole pair table on the device at once:
   orientations of every pair to one of 2^k partitions by the top bits of its record-order hash (glove_cooc_route) and
   merges them into that partition's accumulator (glove_cooc_merge); each partition is then finished on its own
   (glove_cooc_finish_sorted) and, in ascending partition order, its records are formatted into csv lines on the device
-  (glove_cooc_csv_*) and written by a thread while the next block is formatted.
+  (glove_cooc_csv_*) and written by a thread while the next block is formatted.  With ``--format stanford`` / ``both``
+  the same records also go out as Stanford GloVe's binary cooccurrence.shuf.bin (glove_cooc_bin_format).
 
 The device must hold the pair table: about 24 bytes per directed pair plus one merge workspace.  A table that does not
 fit is refused with the figure (DESIGN.md §3, "Streamed corpus preprocessing")."""
+import contextlib
 import csv
 import ctypes
 import io
@@ -43,6 +45,7 @@ _SPACE[[0x09, 0x0a, 0x0b, 0x0c, 0x0d, 0x20, 0x1c, 0x1d, 0x1e, 0x1f]] = True
 _UNICODE_SPACE = re.compile(rb"\xc2[\x85\xa0]|\xe1\x9a\x80|\xe2\x80[\x80-\x8a\xa8\xa9\xaf]|\xe2\x81\x9f|\xe3\x80\x80")
 _PAIR_BYTES = 24                                  # one accumulated directed pair: u64 key + {count, numer}
 _MAX_PART_BITS = 12
+FORMATS = ("csv", "stanford", "both")             # table containers preprocess() writes
 
 
 def text_chunks(path, chunk_bytes, bufs):
@@ -287,27 +290,57 @@ class _Pairs:
         return [t[:got.value] for t in out]
 
 
-class _CsvWriter:
-    """interaction.csv: header, then blocks of records formatted on the device, copied to pinned memory and written by a
-    thread while the next block is formatted."""
+class _PinnedWriter:
+    """Writes device bytes to a file: each block is copied to one of two pinned buffers and written by a thread while
+    the device prepares the next one."""
+
+    def __init__(self, d, f):
+        self.d, self.f = d, f
+        self.pinned, self.pending, self.k = [None, None], [None, None], 0
+        self.pool = ThreadPoolExecutor(max_workers=1)
+        self.bytes = 0
+
+    def _write(self, buf, nbytes, ev):
+        ev.synchronize()
+        self.f.write(buf.numpy()[:nbytes].data)
+
+    def put(self, data, nbytes):
+        """Queues data[:nbytes] (a device tensor of uint8, ready once the current stream reaches this point)."""
+        torch = self.d.torch
+        s = self.k % 2
+        self.k += 1
+        if self.pending[s] is not None:
+            self.pending[s].result()           # the writer is done with this pinned buffer
+        if self.pinned[s] is None or self.pinned[s].numel() < nbytes:
+            self.pinned[s] = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
+        self.pinned[s][:nbytes].copy_(data[:nbytes], non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record()
+        self.pending[s] = self.pool.submit(self._write, self.pinned[s], nbytes, ev)
+        self.bytes += nbytes
+
+    def close(self):
+        try:
+            for p in self.pending:
+                if p is not None:
+                    p.result()
+        finally:
+            self.pool.shutdown(wait=True)
+
+
+class _CsvWriter(_PinnedWriter):
+    """interaction.csv: header, then blocks of records formatted on the device."""
 
     def __init__(self, d, f, vocab_tokens):
+        super().__init__(d, f)
         torch = d.torch
-        self.d, self.f = d, f
         quoted = [csv_quote(t).encode("utf8") for t in vocab_tokens]
         off = np.zeros(len(quoted) + 1, np.int64)
         np.cumsum([len(q) for q in quoted], out=off[1:])
         self.tok = torch.frombuffer(bytearray(b"".join(quoted)), dtype=torch.uint8).to(d.dev)
         self.tok_off = torch.from_numpy(off).to(d.dev)
         self.text = d.empty(0, torch.uint8)
-        self.pinned, self.pending, self.k = [None, None], [None, None], 0
-        self.pool = ThreadPoolExecutor(max_workers=1)
-        self.bytes = 0
         f.write((",".join(COLUMNS) + "\n").encode())
-
-    def _write(self, buf, nbytes, ev):
-        ev.synchronize()
-        self.f.write(buf.numpy()[:nbytes].data)
 
     def write(self, cols, records_per_block):
         d, torch, lib, check = self.d, self.d.torch, self.d.lib, self.d.check
@@ -326,32 +359,42 @@ class _CsvWriter:
                 self.text = d.empty(nbytes, torch.uint8)
             check(lib.glove_cooc_csv_format(*ptrs, n, self.tok.data_ptr(), self.tok_off.data_ptr(), ws.data_ptr(), ws.numel(),
                                             self.text.data_ptr(), self.text.numel(), st), "glove_cooc_csv_format")
-            s = self.k % 2
-            self.k += 1
-            if self.pending[s] is not None:
-                self.pending[s].result()           # the writer is done with this pinned buffer
-            if self.pinned[s] is None or self.pinned[s].numel() < nbytes:
-                self.pinned[s] = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
-            self.pinned[s][:nbytes].copy_(self.text[:nbytes], non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record()
-            self.pending[s] = self.pool.submit(self._write, self.pinned[s], nbytes, ev)
-            self.bytes += nbytes
+            self.put(self.text, nbytes)
 
-    def close(self):
-        try:
-            for p in self.pending:
-                if p is not None:
-                    p.result()
-        finally:
-            self.pool.shutdown(wait=True)
+
+class _BinWriter(_PinnedWriter):
+    """cooccurrence.shuf.bin: Stanford GloVe's 16-byte records (ids + 1, float64 value), formatted on the device in
+    blocks of records (glove_cooc_bin_format)."""
+
+    def __init__(self, d, f):
+        super().__init__(d, f)
+        self.recs = d.empty(0, d.torch.uint8)
+
+    def write(self, cols, records_per_block):
+        d, torch, lib, check = self.d, self.d.torch, self.d.lib, self.d.check
+        st = torch.cuda.current_stream().cuda_stream
+        row, col, value = cols[0], cols[1], cols[3]
+        n_all = len(row)
+        for r0 in range(0, n_all, records_per_block):
+            n = min(records_per_block, n_all - r0)
+            if self.recs.numel() < 16 * n:
+                self.recs = None
+                self.recs = d.empty(16 * n, torch.uint8)
+            check(lib.glove_cooc_bin_format(row[r0:].data_ptr(), col[r0:].data_ptr(), value[r0:].data_ptr(), n,
+                                            self.recs.data_ptr(), st), "glove_cooc_bin_format")
+            self.put(self.recs, 16 * n)
 
 
 def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_size=CONTEXT_SIZE, device="cuda:0",
                chunk_bytes=256 << 20, chunk_positions=16 << 20, partition_entries=1 << 27, records_per_block=1 << 22,
-               order_key=0, device_bytes=None, stats=None):
+               order_key=0, device_bytes=None, stats=None, format="csv"):
     """Writes ``<dest>/vocab.csv``, ``vocab.txt`` and ``interaction.csv`` for the corpus file ``corpus``, byte for byte as
     ``text8.save_data(text8.process_data(text))`` does.  Returns ``(vocabulary frame, number of interaction records)``.
+
+    ``format``: ``"csv"`` (the above), ``"stanford"`` or ``"both"``.  The last two also write the table as Stanford
+    GloVe's ``cooccurrence.shuf.bin`` (16-byte records ``int32 word1, int32 word2, float64 value``, ids 1-based lines of
+    vocab.txt, in interaction.csv's record order) and ``vocab.stanford.txt`` (``token count`` lines in vocab.txt order);
+    ``"stanford"`` writes no interaction.csv.
 
     ``chunk_bytes``: text read per chunk (< 1 GiB); ``chunk_positions``: token positions per pair-counting block;
     ``partition_entries``: target directed pairs per partition of the table (the partition count follows from it and the
@@ -361,6 +404,8 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
     from .text8 import _frame_from_counts
     if not 1 <= int(context_size) <= 8:
         raise ValueError("context_size must be 1..8")
+    if format not in FORMATS:
+        raise ValueError("format must be one of %s, got %r" % (", ".join(FORMATS), format))
     if os.path.getsize(corpus) == 0:
         raise ValueError("%s: empty corpus" % corpus)
     d = _Device(device, device_bytes)
@@ -381,6 +426,9 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
         df_vocab.to_csv(os.path.join(dest, "vocab.csv"), index=False)
         with open(os.path.join(dest, "vocab.txt"), "w") as f:
             f.write("\n".join(df_vocab["token"]))
+        if format != "csv":
+            with open(os.path.join(dest, "vocab.stanford.txt"), "w", encoding="utf8") as f:
+                f.writelines("%s %d\n" % (t, c) for t, c in zip(df_vocab["token"], df_vocab["count"].tolist()))
 
         t1 = time.perf_counter()
         with torch.profiler.record_function("corpus.pass2"):
@@ -431,19 +479,25 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
         t2 = time.perf_counter()
         with torch.profiler.record_function("corpus.write"):
             n_records = 0
-            with open(os.path.join(dest, "interaction.csv"), "wb") as f:
-                writer = _CsvWriter(d, f, vocab_tokens)
-                try:
-                    for p in range(1 << part_bits):
-                        if pairs.n[p] == 0:
-                            continue
-                        cols = pairs.finish(p, vocab_count, total, ctx)
-                        n_records += len(cols[0])
-                        writer.write(cols, int(records_per_block))
-                        del cols
-                finally:
-                    writer.close()
-        stats.update(write_s=time.perf_counter() - t2, records=n_records, csv_bytes=writer.bytes)
+            with contextlib.ExitStack() as files:
+                writers = []
+                if format != "stanford":
+                    writers.append(_CsvWriter(d, files.enter_context(open(os.path.join(dest, "interaction.csv"), "wb")),
+                                              vocab_tokens))
+                    files.callback(writers[-1].close)
+                if format != "csv":
+                    writers.append(_BinWriter(d, files.enter_context(open(os.path.join(dest, "cooccurrence.shuf.bin"), "wb"))))
+                    files.callback(writers[-1].close)
+                for p in range(1 << part_bits):
+                    if pairs.n[p] == 0:
+                        continue
+                    cols = pairs.finish(p, vocab_count, total, ctx)
+                    n_records += len(cols[0])
+                    for w in writers:
+                        w.write(cols, int(records_per_block))
+                    del cols
+        stats.update(write_s=time.perf_counter() - t2, records=n_records,
+                     **{"csv_bytes" if isinstance(w, _CsvWriter) else "bin_bytes": w.bytes for w in writers})
     logger.info("interaction records: %d.", n_records)
     return df_vocab, n_records
 
@@ -456,10 +510,13 @@ def main(argv=None):
     ap.add_argument("--vocab-size", type=int, default=VOCAB_SIZE, help="maximum size of vocab (default: %(default)s)")
     ap.add_argument("--coverage", type=float, default=COVERAGE, help="token coverage to set token count cutoff (default: %(default)s)")
     ap.add_argument("--context-size", type=int, default=CONTEXT_SIZE, help="size of context window (default: %(default)s)")
+    ap.add_argument("--format", default="csv", choices=FORMATS,
+                    help="csv: interaction.csv; stanford: Stanford GloVe's cooccurrence.shuf.bin and vocab.stanford.txt "
+                         "instead; both: all three (default: %(default)s)")
     ap.add_argument("--device", default="cuda:0")
     args = ap.parse_args(argv)
     logger.info("call: %s.", " ".join(sys.argv))
-    preprocess(args.corpus, args.dest, args.vocab_size, args.coverage, args.context_size, args.device)
+    preprocess(args.corpus, args.dest, args.vocab_size, args.coverage, args.context_size, args.device, format=args.format)
 
 
 if __name__ == "__main__":

@@ -8,6 +8,7 @@ device-resident COO triple buffer the trainer shuffles and batches from.  A bina
 parse.  The host only reads the header record and moves bytes."""
 import ctypes
 import os
+import re
 
 import numpy as np
 
@@ -263,6 +264,91 @@ def load_interaction_csv(train_csv, vocab_txt, row_name="row_token", col_name="c
             except OSError:
                 pass
     check_ids(out["row"], out["col"], n_vocab, train_csv)
+    return out
+
+
+COOC_RECORD = 16    # Stanford GloVe co-occurrence record: int32 word1, int32 word2, float64 val (little-endian, packed)
+_STANFORD_LINE = re.compile(r"(\S+) ([0-9]+)")
+
+
+def read_stanford_vocab(vocab_txt):
+    """(tokens, counts) of a vocabulary file.  A file whose first line is ``word count`` (Stanford GloVe's vocab.txt, as
+    vocab_count writes it) must have that form on every line; ``counts`` is then an int64 array.  Any other file is one
+    token per line (``read_vocab``) and ``counts`` is None."""
+    lines = read_vocab(vocab_txt)
+    if not lines or _STANFORD_LINE.fullmatch(lines[0]) is None:
+        return lines, None
+    tokens, counts = [], []
+    for i, line in enumerate(lines):
+        m = _STANFORD_LINE.fullmatch(line)
+        if m is None:
+            raise ValueError("%s: line %d is not 'word count' like line 1: %r" % (vocab_txt, i + 1, line[:80]))
+        tokens.append(m.group(1))
+        counts.append(int(m.group(2)))
+    return tokens, np.array(counts, np.int64)
+
+
+def _bad_record(path, host_rec, g, kind, V):
+    from . import _lib
+    rec = np.frombuffer(host_rec, np.dtype([("w1", "<i4"), ("w2", "<i4"), ("val", "<f8")]))[0]
+    what = {_lib.CREC_BAD_WORD1: "word1 id %d outside 1..%d" % (rec["w1"], V),
+            _lib.CREC_BAD_WORD2: "word2 id %d outside 1..%d" % (rec["w2"], V),
+            _lib.CREC_BAD_VALUE: "val %r is not a finite value > 0" % float(rec["val"])}[kind]
+    return ValueError("%s: record %d (byte %d): %s" % (path, g + 1, g * COOC_RECORD, what))
+
+
+def load_cooc_bin(path, vocab_size, x_max=100.0, alpha=0.75, device="cuda:0", chunk_bytes=64 << 20):
+    """A Stanford GloVe co-occurrence file (cooccurrence.bin or cooccurrence.shuf.bin) as device tensors
+    {'row': i32[n], 'col': i32[n], 'glove_value': f32[n], 'glove_weight': f32[n]} in file order: ids - 1,
+    log(val) and the weight of Stanford's glove.c, ``val >= x_max ? 1 : (val / x_max) ** alpha``, both computed in
+    float64 and rounded once to float32 (csrc/glove_crec.cu).
+
+    The COO is allocated once (the record count follows from the file size) and the chunks, whole records each, are
+    parsed straight into it while reader threads fill the other pinned buffer.  An id outside 1..vocab_size, a val that
+    is not finite and > 0, or a file cut inside a record fails, naming the lowest offending 1-based record and its byte
+    offset."""
+    import torch
+    from . import _lib
+    lib, check = _lib.lib, _lib.check
+    V = int(vocab_size)
+    if not 1 <= V < (1 << 31):
+        raise ValueError("vocab_size must be 1 .. 2^31-1, got %d" % V)
+    size = os.path.getsize(path)
+    n = size // COOC_RECORD
+    dev = torch.device(device)
+    with torch.cuda.device(dev):
+        out = {"row": torch.empty(n, dtype=torch.int32, device=dev), "col": torch.empty(n, dtype=torch.int32, device=dev),
+               "glove_value": torch.empty(n, dtype=torch.float32, device=dev),
+               "glove_weight": torch.empty(n, dtype=torch.float32, device=dev)}
+        if n:
+            st = torch.cuda.current_stream().cuda_stream
+            whole = n * COOC_RECORD
+            chunk = int(max(COOC_RECORD, min(chunk_bytes, whole))) // COOC_RECORD * COOC_RECORD
+            pinned = [torch.empty(_HEAD + chunk, dtype=torch.uint8, pin_memory=True) for _ in range(2 if whole > chunk else 1)]
+            host = [t.numpy() for t in pinned]
+            raw = torch.empty(chunk, dtype=torch.uint8, device=dev)
+            err = torch.full((1,), -1, dtype=torch.int64, device=dev)      # all ones: no bad record
+            reader = _ChunkReader(path, 0, whole, chunk, host * (2 // len(host)))
+            try:
+                reader.start(0)
+                for k in range(reader.n_chunks()):
+                    nb = reader.wait(k)
+                    reader.start(k + 1)
+                    m, first = nb // COOC_RECORD, k * (chunk // COOC_RECORD)
+                    raw[:nb].copy_(pinned[k % len(pinned)][_HEAD:_HEAD + nb], non_blocking=True)
+                    check(lib.glove_cooc_bin_parse(raw.data_ptr(), m, first, V, float(x_max), float(alpha),
+                                                   *[out[c][first:].data_ptr() for c in ("row", "col", "glove_value", "glove_weight")],
+                                                   err.data_ptr(), st), "glove_cooc_bin_parse")
+                    code = int(err.item()) & 0xFFFFFFFFFFFFFFFF       # synchronises: pinned[k % 2] may be refilled after this
+                    if code != 0xFFFFFFFFFFFFFFFF:
+                        g = code >> 2
+                        o = _HEAD + (g - first) * COOC_RECORD
+                        raise _bad_record(path, host[k % len(host)][o:o + COOC_RECORD].tobytes(), g, code & 3, V)
+            finally:
+                reader.close()
+    if size % COOC_RECORD:
+        raise ValueError("%s: record %d (byte %d): the file ends %d bytes into a %d-byte record (truncated file)"
+                         % (path, n + 1, n * COOC_RECORD, size % COOC_RECORD, COOC_RECORD))
     return out
 
 

@@ -1,6 +1,7 @@
 """``python -m glove_tensorflow_b200.estimator`` -- drop-in for ``python -m src.models.estimator`` (ref Makefile:93-98,
 src/models/estimator.py:79-95): same flags, same inputs (interaction.csv + vocab.txt), same job-dir artefacts
-(params.json, vocab.txt copy, checkpoints), the GloVe weighted-least-squares head (RegressionHead with weight column)."""
+(params.json, vocab.txt copy, checkpoints), the GloVe weighted-least-squares head (RegressionHead with weight column).
+``--train-cooc`` trains from a Stanford GloVe cooccurrence.bin instead (data_utils.load_cooc_bin)."""
 import logging
 
 from . import config_utils, data_utils, train_utils
@@ -9,14 +10,23 @@ HEAD = "glove"
 
 
 def build_engine(params, head=HEAD, value_names=None, load_coo=True):
-    """``load_coo=False``: tables only (PREDICT needs the checkpoint and vocab.txt, not interaction.csv)."""
+    """``load_coo=False``: tables only (PREDICT needs the checkpoint and vocab.txt, not interaction.csv).  With
+    ``params["train_cooc"]`` the COO comes from that Stanford GloVe co-occurrence file (``--train-csv`` is ignored)."""
     from .engine import GloveEngine
+    cooc = params.get("train_cooc")
+    if cooc and head != "glove":
+        raise ValueError("--train-cooc trains the glove head only: a Stanford co-occurrence file has no neg_weight column "
+                         "for the %s head (use --train-csv)" % head)
     value_names = value_names or (params["target_name"], params["weight_name"])
+    vocab_size = data_utils.file_lines(params["vocab_txt"])
     coo = None
-    if load_coo:
+    if load_coo and cooc:
+        coo = data_utils.load_cooc_bin(cooc, vocab_size, params.get("x_max", 100.0), params.get("alpha", 0.75),
+                                       device=params.get("device", "cuda:0"))
+        value_names = ("glove_value", "glove_weight")
+    elif load_coo:
         coo = data_utils.load_interaction_csv(params["train_csv"], params["vocab_txt"], params["row_name"],
                                               params["col_name"], value_names, device=params.get("device", "cuda:0"))
-    vocab_size = data_utils.file_lines(params["vocab_txt"])
     reg_scale = params.get("reg_scale")
     if reg_scale is None:
         reg_scale = 2.0  # estimator.py / logistic_matrix_factorisation.py under TF 2.11 (SURVEY A4)

@@ -492,6 +492,23 @@ int glove_cooc_csv_format(const int32_t *row, const int32_t *col, const int64_t 
 int glove_format_float64(double value, char *out, int32_t capacity, int32_t *length);
 int glove_format_float64_device(const uint64_t *bits, int64_t n, char *out, int32_t *len, void *stream);
 
+/* Stanford GloVe co-occurrence records (cooccurrence.bin / .shuf.bin, real = double): struct { int32 word1, word2;
+ * float64 val; }, little-endian, 16 bytes, ids 1-based lines of the vocabulary.
+ * glove_cooc_bin_parse: n records (device memory, 16-byte aligned; record i has the global 0-based index
+ * first_record + i) -> row[i] = word1 - 1, col[i] = word2 - 1, target[i] = (float)log(val),
+ * weight[i] = (float)(val >= x_max ? 1 : pow(val / x_max, alpha)), computed in float64.  A record with an id outside
+ * 1..V or a val that is not finite and > 0 lowers *error (device word; all ones = none) to
+ * global_index * 4 + GLOVE_CREC_BAD_*, so after the call it names the lowest bad record seen so far.  Asynchronous.
+ * glove_cooc_bin_format: n finished records (row, col, value as from glove_cooc_finish*) -> records (16-byte aligned,
+ * 16 n bytes) with ids + 1.  Asynchronous. */
+#define GLOVE_CREC_BAD_WORD1 0
+#define GLOVE_CREC_BAD_WORD2 1
+#define GLOVE_CREC_BAD_VALUE 2
+int glove_cooc_bin_parse(const void *records, int64_t n, int64_t first_record, int64_t V, double x_max, double alpha,
+                         int32_t *row, int32_t *col, float *target, float *weight, unsigned long long *error, void *stream);
+int glove_cooc_bin_format(const int32_t *row, const int32_t *col, const double *value, int64_t n, void *records,
+                          void *stream);
+
 /* ---- HOST-buffer boundary (end to end): what a non-torch caller of the reference's training path would bind ----- */
 /* Runs K TRAIN steps (K a multiple of args->plan_K, at most 4096) on K*B explicit triples held in HOST memory (pinned
  * recommended) and copies the K losses back to host_losses.  Internally a pipeline over the chunks of plan_K steps:
