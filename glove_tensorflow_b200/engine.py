@@ -34,6 +34,15 @@ def adam_alpha_table(learning_rate: float, n_steps: int, beta1: float = ADAM_BET
             / (np.float32(1) - b1p)).astype(np.float32)
 
 
+_DEVICE_ERRORS = {1: "plan / step mismatch", 2: "non-finite loss (a per-item loss term is NaN, infinite or >= 4e18)",
+                  3: "shard blocks too unbalanced for the snapshot buffer"}
+
+
+def _device_error(flag: int) -> str:
+    """'<flag>: <meaning>' of the sticky error word that the step kernels set in the device scalars."""
+    return "%d: %s" % (flag, _DEVICE_ERRORS.get(flag, "unknown"))
+
+
 def _ptr(t: Optional[torch.Tensor]):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p(0)
 
@@ -286,8 +295,7 @@ class GloveEngine:
         out["g"] = np.float32(sc["g"])
         out["step"] = sc["step"]
         if sc["error"]:
-            raise _lib.GloveError("device-side error flag %d set (1: plan / step mismatch, 2: non-finite loss, 3: shard blocks "
-                                  "too unbalanced for the snapshot buffer)" % sc["error"])
+            raise _lib.GloveError("device-side error flag %s" % _device_error(sc["error"]))
         return out
 
     def row_embeddings(self) -> torch.Tensor:
@@ -1119,8 +1127,10 @@ class GloveEngine:
             losses.append(self.loss_out[idx].cpu().numpy())
             done += chunk
         sc = self.read_scalars()
-        if sc["error"] or sc["step"] != self.host_step:
-            raise _lib.GloveError("device step counter %d != host %d (error flag %d)" % (sc["step"], self.host_step, sc["error"]))
+        if sc["error"]:
+            raise _lib.GloveError("device-side error flag %s after step %d" % (_device_error(sc["error"]), sc["step"]))
+        if sc["step"] != self.host_step:
+            raise _lib.GloveError("device step counter %d != host %d" % (sc["step"], self.host_step))
         return np.concatenate(losses) if losses else np.zeros(0, np.float32)
 
     # ---- predict -------------------------------------------------------------------------------------------------

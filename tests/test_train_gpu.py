@@ -346,12 +346,6 @@ def test_row_sharded_tables_on_one_gpu(world, adam_mode, optimizer, V, exchange)
 
 
 def _run_row_sharded(world, adam_mode, optimizer, V, exchange, d=40):
-    import torch
-    from glove_tensorflow_b200.engine import GloveEngine
-    # "+shared-plans": the plan of chunk c is built by engine c % world alone and every engine copies its slice out of the
-    # builder's buffer (glove_plan_pull_slice) -- results must not change by a bit (compared with the oracle like the rest)
-    shared = exchange.endswith("+shared-plans")
-    exchange = exchange.split("+")[0]
     B, steps, n = 512 if world != 3 else 510, 14, 20000
     coo = make_coo(V, n, 51, hot=0.1)
     batches = np.random.default_rng(52).integers(0, n, (steps, B))
@@ -359,9 +353,25 @@ def _run_row_sharded(world, adam_mode, optimizer, V, exchange, d=40):
     ref = st.copy()
     ref_losses = np.array(o.train(ref, coo, batches, optimizer=optimizer, learning_rate=0.01,
                                   adam_mode="lazy" if adam_mode == "lazy" else "keras_dense"))
+    got, losses = _row_sharded_train(world, adam_mode, optimizer, V, exchange, d, st, coo, batches)
+    for k in ("R", "C", "rb", "cb"):
+        assert _rel(got[k], getattr(ref, k)) < 3e-5, (k, _rel(got[k], getattr(ref, k)))
+    assert np.max(np.abs(np.array(losses) - ref_losses) / np.abs(ref_losses)) < RTOL
+
+
+def _row_sharded_train(world, adam_mode, optimizer, V, exchange, d, st, coo, batches, K=5, lr=0.01):
+    """Trains `st` on (coo, batches) with the tables split over `world` owner engines on one GPU; returns the union of the
+    shards' tables (reference layout) and the per-step losses."""
+    import torch
+    from glove_tensorflow_b200.engine import GloveEngine
+    # "+shared-plans": the plan of chunk c is built by engine c % world alone and every engine copies its slice out of the
+    # builder's buffer (glove_plan_pull_slice) -- results must not change by a bit (compared with the oracle like the rest)
+    shared = exchange.endswith("+shared-plans")
+    exchange = exchange.split("+")[0]
+    steps, B = batches.shape
     engs = []
     for r in range(world):
-        e = GloveEngine(V, d, optimizer=optimizer, adam_mode=adam_mode, learning_rate=0.01, batch_size=B, plan_steps=5,
+        e = GloveEngine(V, d, optimizer=optimizer, adam_mode=adam_mode, learning_rate=lr, batch_size=B, plan_steps=K,
                         max_steps=steps + 8, dp_rank=r, dp_world=world, dp_mode="sharded")
         if world in (3, 8):                                        # frequency-balanced owner map instead of id % world
             e.balance_owners(coo["row"], coo["col"], hot=64)       # (the balance itself is checked in tests/test_dp_gloo.py)
@@ -385,7 +395,7 @@ def _run_row_sharded(world, adam_mode, optimizer, V, exchange, d=40):
         if shared:
             # real ranks meet at a barrier before a round of chunks is pulled; engines called one after the other cannot, so
             # the builds of the rounds that this step (and its plan prefetch) may pull from are issued up front
-            for c in (s // 5, s // 5 + 1):
+            for c in (s // K, s // K + 1):
                 for e in engs:
                     e._ring_build(c // world)
             torch.cuda.synchronize()
@@ -441,13 +451,12 @@ def _run_row_sharded(world, adam_mode, optimizer, V, exchange, d=40):
                 e.shard_finish()
         torch.cuda.synchronize()
         losses.append(float(engs[0].read_scalars()["loss"]))
-    got = {k: np.zeros_like(getattr(ref, k)) for k in ("R", "C", "rb", "cb")}
+    got = {k: np.zeros_like(np.asarray(getattr(st, k), np.float32)) for k in ("R", "C", "rb", "cb")}
     for r, e in enumerate(engs):
         stt = e.get_state()
         ids = e.owned_ids()
         assert len(ids) == len(got["rb"][r::world]) and (world in (3, 8) or np.array_equal(ids, np.arange(r, V, world)))
         for k in got:
             got[k][ids] = stt[k][: len(ids)]
-    for k in got:
-        assert _rel(got[k], getattr(ref, k)) < 3e-5, (k, _rel(got[k], getattr(ref, k)))
-    assert np.max(np.abs(np.array(losses) - ref_losses) / np.abs(ref_losses)) < RTOL
+    got["g"], got["step"] = np.float32(engs[0].read_scalars()["g"]), engs[0].read_scalars()["step"]
+    return got, np.array(losses)
