@@ -134,6 +134,11 @@ SIGNATURES = {
     "glove_tokens_count": (ctypes.c_int, [c_void, c_i64, c_void, c_i64, c_void, c_size, c_void, c_void, c_void, c_i64,
                                           ctypes.POINTER(c_i64), c_void]),
     "glove_tokens_lookup": (ctypes.c_int, [c_void, c_void, c_void, c_i64, c_void, c_i64, c_void, c_void, c_void, c_void]),
+    "glove_text_refused": (ctypes.c_int, [c_void, c_i64, c_i32, c_void, ctypes.POINTER(c_i64), c_void]),
+    "glove_tokens_stream_workspace_bytes": (c_size, [c_i64]),
+    "glove_tokens_stream": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_i64, c_i32, c_u32, c_void, c_i64, c_void, c_void,
+                                           c_void, c_size, c_void, c_i64, ctypes.POINTER(c_i64), ctypes.POINTER(c_u32),
+                                           c_void]),
     "glove_cooc_workspace_bytes": (c_size, [c_i64]),
     "glove_cooc_chunk": (ctypes.c_int, [c_void, c_i64, c_i64, c_i32, c_i32, c_void, c_size, c_void, c_void, c_i64,
                                         ctypes.POINTER(c_i64), c_void]),
@@ -148,6 +153,13 @@ SIGNATURES = {
     "glove_cooc_finish_sorted": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, c_i32, c_i64, c_void, c_i64, ctypes.c_uint64,
                                                 c_void, c_size, c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64,
                                                 ctypes.POINTER(c_i64), c_void]),
+    "glove_cooc_chunk_stanford": (ctypes.c_int, [c_void, c_i64, c_i64, c_i32, c_i32, c_i32, c_void, c_size, c_void, c_void,
+                                                 c_i64, ctypes.POINTER(c_i64), c_void]),
+    "glove_cooc_route_stanford": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, ctypes.c_uint64, c_i32, c_i32, c_void, c_size,
+                                                 c_void, c_void, c_i64, c_void, c_void]),
+    "glove_cooc_finish_stanford": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, c_i32, c_i32, c_void, c_i64, ctypes.c_uint64,
+                                                  c_void, c_size, c_void, c_void, c_void, c_void, c_void, c_void, c_void, c_i64,
+                                                  ctypes.POINTER(c_i64), c_void]),
     "glove_vocab_merge_workspace_bytes": (c_size, [c_i64, c_i64]),
     "glove_vocab_merge": (ctypes.c_int, [c_void, c_i64, c_void, c_void, c_void, c_i64, c_void, c_void, c_void, c_void, c_void,
                                          c_i64, c_void, c_i64, c_i64, c_void, c_size, c_void, c_void, c_void, c_void, c_void,

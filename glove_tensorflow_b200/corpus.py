@@ -17,6 +17,11 @@ whole pair table on the device at once:
   (glove_cooc_csv_*) and written by a thread while the next block is formatted.  With ``--format stanford`` / ``both``
   the same records also go out as Stanford GloVe's binary cooccurrence.shuf.bin (glove_cooc_bin_format).
 
+With ``--scheme stanford`` the same two passes follow Stanford GloVe's vocab_count and cooccur instead and write
+vocab.txt (``word count`` lines) and cooccurrence.shuf.bin: vocabulary by count (ties in byte order), out-of-vocabulary
+words removed from the stream, windows of up to 15 words that never cross a line end, self pairs kept, every pair
+written (DESIGN.md §3, "Stanford GloVe preprocessing").
+
 The device must hold the pair table: about 24 bytes per directed pair plus one merge workspace.  A table that does not
 fit is refused with the figure (DESIGN.md §3, "Streamed corpus preprocessing")."""
 import contextlib
@@ -24,6 +29,7 @@ import csv
 import ctypes
 import io
 import logging
+import math
 import os
 import re
 import sys
@@ -46,6 +52,11 @@ _UNICODE_SPACE = re.compile(rb"\xc2[\x85\xa0]|\xe1\x9a\x80|\xe2\x80[\x80-\x8a\xa
 _PAIR_BYTES = 24                                  # one accumulated directed pair: u64 key + {count, numer}
 _MAX_PART_BITS = 12
 FORMATS = ("csv", "stanford", "both")             # table containers preprocess() writes
+SCHEMES = ("reference", "stanford")               # counting rules: text8.process_data's, or vocab_count + cooccur's
+STANFORD_MAX_WINDOW = 15
+# bytes Stanford's tokenizer glues into tokens but the vocabulary readers split on (glove_text_refused)
+_REFUSED = {0x0b: "a vertical tab", 0x0c: "a form feed", 0x0d: "a carriage return not followed by a line feed",
+            **{b: "the separator byte 0x%02x" % b for b in range(0x1c, 0x20)}}
 
 
 def text_chunks(path, chunk_bytes, bufs):
@@ -156,14 +167,39 @@ def _chunk_loop(d, path, chunk_bytes):
         torch.cuda.current_stream().synchronize()
 
 
-def count_tokens(d, path, chunk_bytes):
-    """Pass 1: (tokens in order of first occurrence, their counts)."""
+def _refuse_bytes(d, path, text, fill, host_text, origin, final, scratch):
+    """Raises ValueError naming the lowest offset of a byte glove_text_refused refuses, or of a non-ASCII separator
+    before it."""
+    first = ctypes.c_int64()
+    nxt = -1
+    if not final and host_text[-1] == 0x0d:          # the byte after the chunk decides a \r at its end
+        with open(path, "rb") as f:
+            f.seek(origin + fill)
+            nxt = f.read(1)[0]
+    d.check(d.lib.glove_text_refused(text.data_ptr(), fill, nxt, scratch.data_ptr(), ctypes.byref(first),
+                                     d.torch.cuda.current_stream().cuda_stream), "glove_text_refused")
+    if first.value < 0:
+        return
+    m = _UNICODE_SPACE.search(host_text[:first.value].tobytes())
+    if m is not None:
+        raise ValueError("%s: byte %d: non-ASCII Unicode whitespace, which str.split() would split on"
+                         % (path, origin + m.start()))
+    raise ValueError("%s: byte %d: %s, which Stanford GloVe's tokenizer would keep inside a token"
+                     % (path, origin + first.value, _REFUSED[int(host_text[first.value])]))
+
+
+def count_tokens(d, path, chunk_bytes, stanford=False):
+    """Pass 1: (tokens in order of first occurrence, their counts), and with ``stanford`` also the file offset of each
+    token's first occurrence; ``stanford`` also refuses the bytes of ``_REFUSED``."""
     torch, lib, check = d.torch, d.lib, d.check
     st = torch.cuda.current_stream().cuda_stream
     g = None                     # global table: hash, count, first, off, len
     n_g, pool_used = 0, 0
     pool = d.empty(1 << 20, torch.uint8)
-    for text, fill, host_text, origin, _ in _chunk_loop(d, path, chunk_bytes):
+    scratch = d.empty(1, torch.int64)
+    for text, fill, host_text, origin, final in _chunk_loop(d, path, chunk_bytes):
+        if stanford:
+            _refuse_bytes(d, path, text, fill, host_text, origin, final, scratch)
         starts, _, n = _scan(d, path, text, fill, host_text, origin)
         if n == 0:
             continue
@@ -189,18 +225,30 @@ def count_tokens(d, path, chunk_bytes):
               "glove_vocab_merge")
         g, n_g, pool_used = out, n_out.value, used.value
     if n_g == 0:
-        return [], np.zeros(0, np.int64)
+        return ([], np.zeros(0, np.int64)) + ((np.zeros(0, np.int64),) if stanford else ())
     _, count, first, off, ln = (t[:n_g].cpu().numpy() for t in g)
     blob = pool[:pool_used].cpu().numpy().tobytes()
     order = np.argsort(first, kind="stable")
     tokens = [blob[s:s + n].decode("utf8") for s, n in zip(off[order].tolist(), ln[order].tolist())]
-    return tokens, count[order]
+    return (tokens, count[order]) + ((first[order],) if stanford else ())
 
 
-def _part_bits(vocab_size, n_tokens, context_size, partition_entries):
+def stanford_vocab(tokens, counts, min_count=1, max_vocab=0):
+    """Stanford vocab_count's vocabulary: the tokens with count >= min_count, by count descending and equal counts in
+    byte order (strcmp), the first max_vocab of them (0: all).  Returns (tokens, int64 counts); a token's id is its
+    rank."""
+    keep = [i for i in range(len(tokens)) if counts[i] >= min_count]
+    keep.sort(key=lambda i: (-int(counts[i]), tokens[i].encode("utf8")))
+    if max_vocab:
+        keep = keep[:max_vocab]
+    return [tokens[i] for i in keep], np.array([counts[i] for i in keep], np.int64)
+
+
+def _part_bits(vocab_size, n_tokens, context_size, partition_entries, diagonal=False):
     """Smallest k such that 2^k partitions of the largest possible table (every position pair distinct, or every
-    ordered pair of vocabulary rows) hold at most ``partition_entries`` directed pairs each."""
-    bound = min(vocab_size * (vocab_size - 1), 2 * n_tokens * context_size)
+    ordered pair of vocabulary rows, the diagonal included when self pairs are kept) hold at most ``partition_entries``
+    directed pairs each."""
+    bound = min(vocab_size * (vocab_size if diagonal else vocab_size - 1), 2 * n_tokens * context_size)
     k = 0
     while (bound >> k) > partition_entries and k < _MAX_PART_BITS:
         k += 1
@@ -208,10 +256,11 @@ def _part_bits(vocab_size, n_tokens, context_size, partition_entries):
 
 
 class _Pairs:
-    """Pass 2 accumulators: one sorted, reduced table of directed pairs per partition."""
+    """Pass 2 accumulators: one sorted, reduced table of directed pairs per partition.  ``stanford``: None for the
+    reference rules, or (window, distance_weighting, symmetric)."""
 
-    def __init__(self, d, V, part_bits, order_key):
-        self.d, self.V, self.part_bits, self.order_key = d, V, part_bits, order_key
+    def __init__(self, d, V, part_bits, order_key, stanford=None):
+        self.d, self.V, self.part_bits, self.order_key, self.stanford = d, V, part_bits, order_key, stanford
         self.acc = [None] * (1 << part_bits)
         self.n = [0] * (1 << part_bits)
         self.ws = d.empty(0, d.torch.uint8)
@@ -238,15 +287,23 @@ class _Pairs:
                                  budget / 1e9))
 
     def add(self, keys, agg, n):
-        """Routes both orientations of a right-context table (n entries) and merges them into the partitions."""
+        """Routes both orientations of a right-context table (n entries), or only (left, right) for an asymmetric
+        Stanford table, and merges them into the partitions."""
         d, torch, lib, check = self.d, self.d.torch, self.d.lib, self.d.check
         st = torch.cuda.current_stream().cuda_stream
         P = 1 << self.part_bits
-        rk, ra = d.empty(2 * n, torch.int64), d.empty(4 * n, torch.int64)
+        n_out = n if self.stanford is not None and not self.stanford[2] else 2 * n
+        rk, ra = d.empty(n_out, torch.int64), d.empty(2 * n_out, torch.int64)
         rws = d.empty(lib.glove_cooc_route_workspace_bytes(n, self.part_bits), torch.uint8)
         counts = np.zeros(P, np.int64)
-        check(lib.glove_cooc_route(keys.data_ptr(), agg.data_ptr(), n, self.V, self.order_key, self.part_bits, rws.data_ptr(),
-                                   rws.numel(), rk.data_ptr(), ra.data_ptr(), 2 * n, counts.ctypes.data, st), "glove_cooc_route")
+        if self.stanford is None:
+            check(lib.glove_cooc_route(keys.data_ptr(), agg.data_ptr(), n, self.V, self.order_key, self.part_bits,
+                                       rws.data_ptr(), rws.numel(), rk.data_ptr(), ra.data_ptr(), n_out, counts.ctypes.data, st),
+                  "glove_cooc_route")
+        else:
+            check(lib.glove_cooc_route_stanford(keys.data_ptr(), agg.data_ptr(), n, self.V, self.order_key, self.part_bits,
+                                                int(self.stanford[2]), rws.data_ptr(), rws.numel(), rk.data_ptr(), ra.data_ptr(),
+                                                n_out, counts.ctypes.data, st), "glove_cooc_route_stanford")
         del rws
         got = ctypes.c_int64()
         o = 0
@@ -283,9 +340,15 @@ class _Pairs:
         dts = (torch.int32, torch.int32, torch.int64, torch.float64, torch.float64, torch.float64, torch.float64)
         out = [d.empty(n, dt) for dt in dts]
         got = ctypes.c_int64()
-        check(lib.glove_cooc_finish_sorted(keys.data_ptr(), agg.data_ptr(), n, self.V, context_size, 10, vocab_count.data_ptr(),
-                                           total, self.order_key, ws.data_ptr(), ws.numel(), *[t.data_ptr() for t in out], n,
-                                           ctypes.byref(got), st), "glove_cooc_finish_sorted")
+        if self.stanford is None:
+            check(lib.glove_cooc_finish_sorted(keys.data_ptr(), agg.data_ptr(), n, self.V, context_size, 10,
+                                               vocab_count.data_ptr(), total, self.order_key, ws.data_ptr(), ws.numel(),
+                                               *[t.data_ptr() for t in out], n, ctypes.byref(got), st), "glove_cooc_finish_sorted")
+        else:
+            check(lib.glove_cooc_finish_stanford(keys.data_ptr(), agg.data_ptr(), n, self.V, context_size,
+                                                 int(self.stanford[1]), vocab_count.data_ptr(), total, self.order_key,
+                                                 ws.data_ptr(), ws.numel(), *[t.data_ptr() for t in out], n, ctypes.byref(got),
+                                                 st), "glove_cooc_finish_stanford")
         self.acc[p], self.n[p] = None, 0
         return [t[:got.value] for t in out]
 
@@ -385,9 +448,58 @@ class _BinWriter(_PinnedWriter):
             self.put(self.recs, 16 * n)
 
 
+def _newline_after_last_token(text, newline_before):
+    """Whether a '\\n' follows the last token of ``text`` (a chunk's own bytes); for a chunk without tokens, whether one
+    lies in it or before it."""
+    i, window = len(text), 4096
+    while i > 0:
+        j = max(0, i - window)
+        hit = np.flatnonzero(~_SPACE[text[j:i]])
+        if len(hit):
+            return bool((text[j + int(hit[-1]) + 1:] == 0x0A).any())
+        i, window = j, window * 16
+    return newline_before or bool((text == 0x0A).any())
+
+
+class _StanfordStream:
+    """Pass 2 of the Stanford scheme: the in-vocabulary tokens of each chunk, in text order, as (line segment << 32) |
+    id (glove_tokens_stream); the segment and the '\\n' after the last token carry over to the next chunk."""
+
+    def __init__(self, d, vocab):
+        self.d, self.vocab = d, vocab
+        self.end, self.newline, self.segment = 0, False, 0
+
+    def ids(self, text, fill, host_text, origin, starts, lens, n):
+        d, torch = self.d, self.d.torch
+        begin = self.end - origin                     # the chunk's own bytes start here (the rest is padding)
+        self.end = origin + fill
+        if n == 0:
+            self.newline = _newline_after_last_token(host_text[begin:], self.newline)
+            return torch.empty(0, dtype=torch.int64, device=d.dev)
+        table, slots, vb, voff = self.vocab
+        ws = d.empty(d.lib.glove_tokens_stream_workspace_bytes(n), torch.uint8)
+        out = d.empty(n, torch.int64)
+        got, last = ctypes.c_int64(), ctypes.c_uint32()
+        d.check(d.lib.glove_tokens_stream(text.data_ptr(), begin, starts.data_ptr(), lens.data_ptr(), n, int(self.newline),
+                                          self.segment, table.data_ptr(), slots, vb.data_ptr(), voff.data_ptr(), ws.data_ptr(),
+                                          ws.numel(), out.data_ptr(), n, ctypes.byref(got), ctypes.byref(last),
+                                          torch.cuda.current_stream().cuda_stream), "glove_tokens_stream")
+        self.segment = last.value
+        self.newline = _newline_after_last_token(host_text[begin:], False)
+        return out[:got.value]
+
+
+def _stanford_numerator_bound(n_tokens, window, distance_weighting, symmetric):
+    """The largest numerator a pair can reach: every position adds at most sum_k w_k per orientation."""
+    unit = math.lcm(*range(1, window + 1))
+    per_position = sum(unit // k for k in range(1, window + 1)) if distance_weighting else window
+    return int(n_tokens) * per_position * (2 if symmetric else 1)
+
+
 def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_size=CONTEXT_SIZE, device="cuda:0",
                chunk_bytes=256 << 20, chunk_positions=16 << 20, partition_entries=1 << 27, records_per_block=1 << 22,
-               order_key=0, device_bytes=None, stats=None, format="csv"):
+               order_key=0, device_bytes=None, stats=None, format="csv", scheme="reference", window_size=15, min_count=1,
+               max_vocab=0, symmetric=True, distance_weighting=True):
     """Writes ``<dest>/vocab.csv``, ``vocab.txt`` and ``interaction.csv`` for the corpus file ``corpus``, byte for byte as
     ``text8.save_data(text8.process_data(text))`` does.  Returns ``(vocabulary frame, number of interaction records)``.
 
@@ -396,13 +508,28 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
     vocab.txt, in interaction.csv's record order) and ``vocab.stanford.txt`` (``token count`` lines in vocab.txt order);
     ``"stanford"`` writes no interaction.csv.
 
+    ``scheme="stanford"`` counts as Stanford GloVe's ``vocab_count -min-count min_count -max-vocab max_vocab`` and
+    ``cooccur -window-size window_size -symmetric symmetric -distance-weighting distance_weighting`` do and writes
+    ``<dest>/vocab.txt`` (``word count`` lines) and ``<dest>/cooccurrence.shuf.bin`` only; ``vocab_size``, ``coverage``,
+    ``context_size`` and ``format`` are then unused.  Returns the vocabulary (columns token, count) and the record
+    count.  The rules are those of DESIGN.md §3, "Stanford GloVe preprocessing".
+
     ``chunk_bytes``: text read per chunk (< 1 GiB); ``chunk_positions``: token positions per pair-counting block;
     ``partition_entries``: target directed pairs per partition of the table (the partition count follows from it and the
     corpus; small values exercise the partitioning); ``device_bytes``: device memory the pair table may use (default:
     what is free).  ``stats``: a dict that receives pass timings and sizes."""
     import time
+    import pandas as pd
     from .text8 import _frame_from_counts
-    if not 1 <= int(context_size) <= 8:
+    if scheme not in SCHEMES:
+        raise ValueError("scheme must be one of %s, got %r" % (", ".join(SCHEMES), scheme))
+    stanford = scheme == "stanford"
+    if stanford:
+        if not 1 <= int(window_size) <= STANFORD_MAX_WINDOW:
+            raise ValueError("window_size must be 1..%d" % STANFORD_MAX_WINDOW)
+        if int(min_count) < 1 or int(max_vocab) < 0:
+            raise ValueError("min_count must be >= 1 and max_vocab >= 0")
+    elif not 1 <= int(context_size) <= 8:
         raise ValueError("context_size must be 1..8")
     if format not in FORMATS:
         raise ValueError("format must be one of %s, got %r" % (", ".join(FORMATS), format))
@@ -415,24 +542,39 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
         st = torch.cuda.current_stream().cuda_stream
         t0 = time.perf_counter()
         with torch.profiler.record_function("corpus.pass1"):
-            tokens, counts = count_tokens(d, corpus, chunk_bytes)
+            tokens, counts, *first = count_tokens(d, corpus, chunk_bytes, stanford)
         n_tokens = int(counts.sum())
         if n_tokens < 2:
             raise ValueError("%s: need at least two tokens, the corpus holds %d" % (corpus, n_tokens))
-        df_vocab = _frame_from_counts(tokens, counts, None if vocab_size is None else int(vocab_size), coverage)
+        os.makedirs(dest, exist_ok=True)
+        if stanford:
+            if "<unk>" in tokens:
+                raise ValueError("%s: byte %d: the token <unk>, which Stanford GloVe reserves"
+                                 % (corpus, int(first[0][tokens.index("<unk>")])))
+            ctx = int(window_size)
+            if _stanford_numerator_bound(n_tokens, ctx, distance_weighting, symmetric) >= 1 << 63:
+                raise ValueError("%s: %d tokens: a pair's exact weight sum could overflow 64 bits" % (corpus, n_tokens))
+            vocab_tokens, vocab_counts = stanford_vocab(tokens, counts, int(min_count), int(max_vocab))
+            if not vocab_tokens:
+                raise ValueError("%s: no token occurs at least %d times" % (corpus, min_count))
+            df_vocab = pd.DataFrame({"token": vocab_tokens, "count": vocab_counts})
+            with open(os.path.join(dest, "vocab.txt"), "w", encoding="utf8") as f:
+                f.writelines("%s %d\n" % (t, c) for t, c in zip(vocab_tokens, vocab_counts.tolist()))
+        else:
+            ctx = int(context_size)
+            df_vocab = _frame_from_counts(tokens, counts, None if vocab_size is None else int(vocab_size), coverage)
+            vocab_tokens = df_vocab["token"].tolist()
+            df_vocab.to_csv(os.path.join(dest, "vocab.csv"), index=False)
+            with open(os.path.join(dest, "vocab.txt"), "w") as f:
+                f.write("\n".join(df_vocab["token"]))
+            if format != "csv":
+                with open(os.path.join(dest, "vocab.stanford.txt"), "w", encoding="utf8") as f:
+                    f.writelines("%s %d\n" % (t, c) for t, c in zip(df_vocab["token"], df_vocab["count"].tolist()))
         logger.info("vocab created, size: %s.", df_vocab.shape[0])
         stats.update(pass1_s=time.perf_counter() - t0, distinct_tokens=len(tokens), tokens=n_tokens)
-        os.makedirs(dest, exist_ok=True)
-        df_vocab.to_csv(os.path.join(dest, "vocab.csv"), index=False)
-        with open(os.path.join(dest, "vocab.txt"), "w") as f:
-            f.write("\n".join(df_vocab["token"]))
-        if format != "csv":
-            with open(os.path.join(dest, "vocab.stanford.txt"), "w", encoding="utf8") as f:
-                f.writelines("%s %d\n" % (t, c) for t, c in zip(df_vocab["token"], df_vocab["count"].tolist()))
 
         t1 = time.perf_counter()
         with torch.profiler.record_function("corpus.pass2"):
-            vocab_tokens = df_vocab["token"].tolist()
             V = len(vocab_tokens)
             lines = [t.encode("utf8") for t in vocab_tokens]
             off = np.zeros(V + 1, np.int64)
@@ -444,17 +586,23 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
             check(lib.glove_vocab_build(table.data_ptr(), slots, vb.data_ptr(), voff.data_ptr(), V, st), "glove_vocab_build")
             vocab_count = torch.from_numpy(np.array(df_vocab["count"], np.int64)).to(d.dev)
             total = int(df_vocab["count"].sum())
-            ctx = int(context_size)
             block = int(max(1, min(chunk_positions, (1 << 28) // ctx)))
-            part_bits = _part_bits(V, n_tokens, ctx, int(partition_entries))
-            pairs = _Pairs(d, V, part_bits, order_key)
+            part_bits = _part_bits(V, n_tokens, ctx, int(partition_entries), diagonal=stanford)
+            pairs = _Pairs(d, V, part_bits, order_key,
+                           (ctx, bool(distance_weighting), bool(symmetric)) if stanford else None)
+            stream = _StanfordStream(d, (table, slots, vb, voff)) if stanford else None
             cws = d.empty(lib.glove_cooc_workspace_bytes(block * ctx), torch.uint8)
             got = ctypes.c_int64()
-            tail = torch.empty(0, dtype=torch.int32, device=d.dev)     # ids whose right context lies in the next chunk
+            # ids (Stanford: (segment << 32) | id) whose right context lies in the next chunk
+            tail = torch.empty(0, dtype=torch.int64 if stanford else torch.int32, device=d.dev)
             for text, fill, host_text, origin, final in _chunk_loop(d, corpus, chunk_bytes):
                 starts, lens, n = _scan(d, corpus, text, fill, host_text, origin)
                 ids = tail
-                if n:
+                if stanford:
+                    new = stream.ids(text, fill, host_text, origin, starts, lens, n)
+                    if new.numel():
+                        ids = torch.cat([tail, new])
+                elif n:
                     ids = torch.empty(tail.numel() + n, dtype=torch.int32, device=d.dev)
                     ids[:tail.numel()].copy_(tail)
                     check(lib.glove_tokens_lookup(text.data_ptr(), starts.data_ptr(), lens.data_ptr(), n, table.data_ptr(), slots,
@@ -467,8 +615,13 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
                     n_t = min(n_p + ctx, T - p0)
                     cap = n_p * ctx
                     k, a = d.empty(cap, torch.int64), d.empty(2 * cap, torch.int64)
-                    check(lib.glove_cooc_chunk(ids[p0:].data_ptr(), n_p, n_t, V, ctx, cws.data_ptr(), cws.numel(), k.data_ptr(),
-                                               a.data_ptr(), cap, ctypes.byref(got), st), "glove_cooc_chunk")
+                    if stanford:
+                        check(lib.glove_cooc_chunk_stanford(ids[p0:].data_ptr(), n_p, n_t, V, ctx, int(distance_weighting),
+                                                            cws.data_ptr(), cws.numel(), k.data_ptr(), a.data_ptr(), cap,
+                                                            ctypes.byref(got), st), "glove_cooc_chunk_stanford")
+                    else:
+                        check(lib.glove_cooc_chunk(ids[p0:].data_ptr(), n_p, n_t, V, ctx, cws.data_ptr(), cws.numel(),
+                                                   k.data_ptr(), a.data_ptr(), cap, ctypes.byref(got), st), "glove_cooc_chunk")
                     if got.value:
                         pairs.add(k, a, got.value)
                     del k, a
@@ -481,11 +634,11 @@ def preprocess(corpus, dest, vocab_size=VOCAB_SIZE, coverage=COVERAGE, context_s
             n_records = 0
             with contextlib.ExitStack() as files:
                 writers = []
-                if format != "stanford":
+                if format != "stanford" and not stanford:
                     writers.append(_CsvWriter(d, files.enter_context(open(os.path.join(dest, "interaction.csv"), "wb")),
                                               vocab_tokens))
                     files.callback(writers[-1].close)
-                if format != "csv":
+                if format != "csv" or stanford:
                     writers.append(_BinWriter(d, files.enter_context(open(os.path.join(dest, "cooccurrence.shuf.bin"), "wb"))))
                     files.callback(writers[-1].close)
                 for p in range(1 << part_bits):
@@ -513,10 +666,23 @@ def main(argv=None):
     ap.add_argument("--format", default="csv", choices=FORMATS,
                     help="csv: interaction.csv; stanford: Stanford GloVe's cooccurrence.shuf.bin and vocab.stanford.txt "
                          "instead; both: all three (default: %(default)s)")
+    ap.add_argument("--scheme", default="reference", choices=SCHEMES,
+                    help="reference: the counting rules of text8.process_data and the files above; stanford: those of "
+                         "Stanford GloVe's vocab_count and cooccur, written as vocab.txt and cooccurrence.shuf.bin "
+                         "(default: %(default)s)")
+    ap.add_argument("--window-size", type=int, default=15,
+                    help="stanford: words of context on each side, 1..%d (default: %%(default)s)" % STANFORD_MAX_WINDOW)
+    ap.add_argument("--min-count", type=int, default=1, help="stanford: least count of a vocabulary word (default: %(default)s)")
+    ap.add_argument("--max-vocab", type=int, default=0, help="stanford: largest vocabulary, 0 for no limit (default: %(default)s)")
+    ap.add_argument("--asymmetric", action="store_true", help="stanford: left context only (cooccur -symmetric 0)")
+    ap.add_argument("--no-distance-weighting", action="store_true",
+                    help="stanford: every pair counts 1 instead of 1/distance (cooccur -distance-weighting 0)")
     ap.add_argument("--device", default="cuda:0")
     args = ap.parse_args(argv)
     logger.info("call: %s.", " ".join(sys.argv))
-    preprocess(args.corpus, args.dest, args.vocab_size, args.coverage, args.context_size, args.device, format=args.format)
+    preprocess(args.corpus, args.dest, args.vocab_size, args.coverage, args.context_size, args.device, format=args.format,
+               scheme=args.scheme, window_size=args.window_size, min_count=args.min_count, max_vocab=args.max_vocab,
+               symmetric=not args.asymmetric, distance_weighting=not args.no_distance_weighting)
 
 
 if __name__ == "__main__":

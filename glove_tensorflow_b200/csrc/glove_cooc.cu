@@ -13,6 +13,11 @@
 //                 [ref text8.py:130-139]; records come out in a keyed-hash order (the reference orders them by Python's
 //                 per-process salted hash() of the token pair, i.e. randomly [ref text8.py:119-124])
 //
+// The Stanford GloVe scheme (vocab_count / cooccur, corpus.py scheme "stanford") shares the sort, reduce, route and
+// finish code: emit_line_pairs_kernel emits (left, right) at distances 1..window (<= 15) within one line of the
+// in-vocabulary token stream, self pairs kept, weights lcm(1..window)/k or 1; route sends one or both orientations;
+// every pair becomes a record.
+//
 // Integer / sort work, HBM-bound: CUB radix sort + reduce-by-key around small hand-written kernels; no tensor cores.
 #include <cub/cub.cuh>
 #include <thrust/iterator/transform_iterator.h>
@@ -29,11 +34,15 @@ struct AggSum {
         return Agg{a.count + b.count, a.numer + b.numer};
     }
 };
-// payload k-1 of a sorted pair -> its contribution {1, L/k}
-struct KToAgg {
-    long long w[8];
-    __host__ __device__ __forceinline__ Agg operator()(const uint8_t &k1) const { return Agg{1, w[k1 & 7]}; }
+// payload k-1 of a sorted pair -> its contribution {1, w[k-1]}; N = 8 (reference contexts 1..8) or 16 (Stanford windows
+// 1..15), so that the reference pass carries no more payload table than it needs
+template <int N> struct KToAggN {
+    long long w[N];
+    __host__ __device__ __forceinline__ Agg operator()(const uint8_t &k1) const { return Agg{1, w[k1 & (N - 1)]}; }
 };
+using KToAgg = KToAggN<8>;
+using KToAgg16 = KToAggN<16>;
+constexpr int kStanfordMaxWindow = 15;
 
 static int vbits_of(int64_t V) {
     int b = 1;
@@ -79,6 +88,10 @@ static CoocWs cooc_ws_view(void *base, int64_t n) {
     cub::DeviceRadixSort::SortPairs(nullptr, b, (uint64_t *)nullptr, (uint64_t *)nullptr, (uint32_t *)nullptr, (uint32_t *)nullptr, ni);
     thrust::transform_iterator<KToAgg, const uint8_t *> it((const uint8_t *)nullptr, KToAgg());
     cub::DeviceReduce::ReduceByKey(nullptr, c, (uint64_t *)nullptr, (uint64_t *)nullptr, it, (Agg *)nullptr, (long long *)nullptr, AggSum(), ni);
+    size_t c16 = 0;
+    thrust::transform_iterator<KToAgg16, const uint8_t *> it16((const uint8_t *)nullptr, KToAgg16());
+    cub::DeviceReduce::ReduceByKey(nullptr, c16, (uint64_t *)nullptr, (uint64_t *)nullptr, it16, (Agg *)nullptr, (long long *)nullptr, AggSum(), ni);
+    if (c16 > c) c = c16;
     cub::DeviceReduce::ReduceByKey(nullptr, d, (uint64_t *)nullptr, (uint64_t *)nullptr, (Agg *)nullptr, (Agg *)nullptr, (long long *)nullptr, AggSum(), ni);
     cub::DeviceSelect::Flagged(nullptr, e, (uint32_t *)nullptr, (uint8_t *)nullptr, (uint32_t *)nullptr, (long long *)nullptr, ni);
     w.cub_bytes = a;
@@ -105,6 +118,27 @@ __global__ void __launch_bounds__(256) emit_pairs_kernel(const int32_t *__restri
         const int32_t a = ids[p], b = ids[p + k];
         if (a < 0 || a >= V || b < 0 || b >= V) *bad = 1;
         else if (a != b) key = ((uint64_t)(uint32_t)a << vbits) | (uint32_t)b;
+    }
+    keys[t] = key;
+    kk[t] = (uint8_t)(k - 1);
+}
+
+// Stanford GloVe's cooccur: pair (p, k): left = id of tok[p], right = id of tok[p + k], emitted only when both lie on one
+// line (equal segment ids); self pairs are kept.  tok[i] = (segment << 32) | id, the in-vocabulary tokens in text order
+// (glove_tokens_stream), so out-of-vocabulary words take no position.
+__global__ void __launch_bounds__(256) emit_line_pairs_kernel(const uint64_t *__restrict__ tok, int64_t n_positions,
+                                                              int64_t n_tokens, int32_t window, int vbits, int32_t V,
+                                                              uint64_t *keys, uint8_t *kk, int32_t *bad) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_positions * window) return;
+    const int64_t p = t / window;
+    const int k = (int)(t - p * window) + 1;
+    uint64_t key = (1ull << (2 * vbits)) - 1;          // as in emit_pairs_kernel: never a valid pair, sorts last
+    if (p + k < n_tokens) {
+        const uint64_t x = tok[p], y = tok[p + k];
+        const int32_t a = (int32_t)(uint32_t)x, b = (int32_t)(uint32_t)y;
+        if (a < 0 || a >= V || b < 0 || b >= V) *bad = 1;
+        else if ((x >> 32) == (y >> 32)) key = ((uint64_t)(uint32_t)a << vbits) | (uint32_t)b;
     }
     keys[t] = key;
     kk[t] = (uint8_t)(k - 1);
@@ -180,19 +214,19 @@ __device__ __forceinline__ uint64_t directed_key(const uint64_t *keys, int64_t n
     const uint64_t k = keys[t < n ? t : t - n], mask = (1ull << vbits) - 1;
     return t < n ? k : ((k & mask) << vbits) | (k >> vbits);
 }
-// t < n: entry t as (a, b); t >= n: entry t - n as (b, a)
-__global__ void __launch_bounds__(256) route_parts_kernel(const uint64_t *__restrict__ keys, int64_t n, int vbits, uint64_t salt,
-                                                          int part_bits, uint32_t *part, uint32_t *idx) {
+// t < n: entry t as (a, b); t >= n: entry t - n as (b, a); n_orient = 2 routes both orientations, 1 only (a, b)
+__global__ void __launch_bounds__(256) route_parts_kernel(const uint64_t *__restrict__ keys, int64_t n, int n_orient, int vbits,
+                                                          uint64_t salt, int part_bits, uint32_t *part, uint32_t *idx) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 2 * n) return;
+    if (t >= n_orient * n) return;
     part[t] = part_of(directed_key(keys, n, t, vbits), salt, part_bits);
     idx[t] = (uint32_t)t;
 }
 __global__ void __launch_bounds__(256) route_scatter_kernel(const uint64_t *__restrict__ keys, const Agg *__restrict__ agg,
-                                                            int64_t n, int vbits, const uint32_t *__restrict__ order,
+                                                            int64_t n, int n_orient, int vbits, const uint32_t *__restrict__ order,
                                                             uint64_t *out_keys, Agg *out_agg) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= 2 * n) return;
+    if (i >= n_orient * n) return;
     const int64_t t = order[i];
     out_keys[i] = directed_key(keys, n, t, vbits);
     out_agg[i] = agg[t < n ? t : t - n];
@@ -226,6 +260,77 @@ static RouteWs route_ws_view(void *base, int64_t n2, int part_bits) {
 static int read_count(const long long *dev, long long *host, cudaStream_t stream) {
     GLOVE_CHECK_CUDA(cudaMemcpyAsync(host, dev, sizeof(long long), cudaMemcpyDeviceToHost, stream));
     GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    return GLOVE_OK;
+}
+
+// sorts the n emitted (key, k-1) pairs of a chunk and reduces them to {count, sum of w[k-1]} per key into the caller's
+// buffers, dropping the sentinel run
+template <class Conv>
+static int reduce_chunk_pairs(const char *who, const CoocWs &w, int64_t n, int vbits, const Conv &conv, int32_t V,
+                              const int32_t *bad, uint64_t *out_keys, int64_t *out_agg, int64_t capacity,
+                              int64_t *n_unique_host, cudaStream_t stream) {
+    size_t tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.keys[0], w.keys[1], w.kk[0], w.kk[1], (int)n, 0,
+                                                     2 * vbits, stream));
+    thrust::transform_iterator<Conv, const uint8_t *> vals(w.kk[1], conv);
+    tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceReduce::ReduceByKey(w.cub_temp, tb, w.keys[1], w.keys[0], vals, w.agg, w.count_out, AggSum(),
+                                                    (int)n, stream));
+    long long runs = 0;
+    int32_t bad_h = 0;
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(&bad_h, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    if (int rc = read_count(w.count_out, &runs, stream)) return rc;
+    if (bad_h) return set_error(GLOVE_EINVAL, "%s: token id outside [0, %d)", who, V);
+    // the sentinel run (dropped pairs), when present, is the last one
+    uint64_t last_key = 0;
+    if (runs > 0) {
+        GLOVE_CHECK_CUDA(cudaMemcpyAsync(&last_key, w.keys[0] + runs - 1, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+        if (last_key == (1ull << (2 * vbits)) - 1) --runs;
+    }
+    if (runs > capacity)
+        return set_error(GLOVE_EINVAL, "%s: %lld distinct pairs > capacity %lld", who, runs, (long long)capacity);
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(out_keys, w.keys[0], sizeof(uint64_t) * runs, cudaMemcpyDeviceToDevice, stream));
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(out_agg, w.agg, sizeof(Agg) * runs, cudaMemcpyDeviceToDevice, stream));
+    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    *n_unique_host = runs;
+    return GLOVE_OK;
+}
+
+// routes n_orient orientations of every entry of a table to its partition (glove_cooc_route*); arguments checked
+static int route_entries(const char *who, const uint64_t *keys, const int64_t *agg, int64_t n, int n_orient, int32_t V,
+                         uint64_t order_key, int32_t part_bits, void *workspace, size_t workspace_bytes, uint64_t *out_keys,
+                         int64_t *out_agg, int64_t *part_count_host, cudaStream_t stream) {
+    const int vbits = vbits_of((int64_t)V + 1);
+    const int64_t n2 = n_orient * n;
+    const RouteWs w = route_ws_view(workspace, n2, part_bits);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "%s: workspace %zu < required %zu", who, workspace_bytes, w.bytes);
+    const unsigned g = (unsigned)((n2 + 255) / 256);
+    route_parts_kernel<<<g, 256, 0, stream>>>(keys, n, n_orient, vbits, order_key, part_bits, w.part[0], w.idx[0]);
+    GLOVE_CHECK_LAUNCH();
+    const uint32_t *order = w.idx[0];
+    const int P = 1 << part_bits;
+    if (part_bits) {
+        size_t tb = w.cub_bytes;
+        GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.part[0], w.part[1], w.idx[0], w.idx[1], (int)n2, 0,
+                                                         part_bits, stream));
+        tb = w.cub_bytes;
+        GLOVE_CHECK_CUDA(cub::DeviceHistogram::HistogramEven(w.cub_temp, tb, w.part[1], w.hist, P + 1, 0u, (uint32_t)P, (int)n2,
+                                                             stream));
+        order = w.idx[1];
+    }
+    route_scatter_kernel<<<g, 256, 0, stream>>>(keys, (const Agg *)agg, n, n_orient, vbits, order, out_keys, (Agg *)out_agg);
+    GLOVE_CHECK_LAUNCH();
+    if (part_bits) {
+        int hist[1 << kCoocMaxPartBits];
+        GLOVE_CHECK_CUDA(cudaMemcpyAsync(hist, w.hist, sizeof(int) * P, cudaMemcpyDeviceToHost, stream));
+        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+        for (int p = 0; p < P; ++p) part_count_host[p] = hist[p];
+    } else {
+        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+        part_count_host[0] = n2;
+    }
     return GLOVE_OK;
 }
 
@@ -291,35 +396,36 @@ int glove_cooc_chunk(const int32_t *token_ids, int64_t n_positions, int64_t n_to
     emit_pairs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(token_ids, n_positions, n_tokens, context, vbits, V,
                                                                         w.keys[0], w.kk[0], bad);
     GLOVE_CHECK_LAUNCH();
-    size_t tb = w.cub_bytes;
-    GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.keys[0], w.keys[1], w.kk[0], w.kk[1], (int)n, 0,
-                                                     2 * vbits, stream));
     KToAgg conv;
     const long long unit = lcm_upto(context);
     for (int k = 0; k < 8; ++k) conv.w[k] = k < context ? unit / (k + 1) : 0;
-    thrust::transform_iterator<KToAgg, const uint8_t *> vals(w.kk[1], conv);
-    tb = w.cub_bytes;
-    GLOVE_CHECK_CUDA(cub::DeviceReduce::ReduceByKey(w.cub_temp, tb, w.keys[1], w.keys[0], vals, w.agg, w.count_out, AggSum(),
-                                                    (int)n, stream));
-    long long runs = 0;
-    int32_t bad_h = 0;
-    GLOVE_CHECK_CUDA(cudaMemcpyAsync(&bad_h, bad, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
-    if (int rc = read_count(w.count_out, &runs, stream)) return rc;
-    if (bad_h) return set_error(GLOVE_EINVAL, "glove_cooc_chunk: token id outside [0, %d)", V);
-    // the sentinel run (dropped pairs), when present, is the last one
-    uint64_t last_key = 0;
-    if (runs > 0) {
-        GLOVE_CHECK_CUDA(cudaMemcpyAsync(&last_key, w.keys[0] + runs - 1, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
-        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
-        if (last_key == (1ull << (2 * vbits)) - 1) --runs;
-    }
-    if (runs > capacity)
-        return set_error(GLOVE_EINVAL, "glove_cooc_chunk: %lld distinct pairs > capacity %lld", runs, (long long)capacity);
-    GLOVE_CHECK_CUDA(cudaMemcpyAsync(out_keys, w.keys[0], sizeof(uint64_t) * runs, cudaMemcpyDeviceToDevice, stream));
-    GLOVE_CHECK_CUDA(cudaMemcpyAsync(out_agg, w.agg, sizeof(Agg) * runs, cudaMemcpyDeviceToDevice, stream));
-    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
-    *n_unique_host = runs;
-    return GLOVE_OK;
+    return reduce_chunk_pairs("glove_cooc_chunk", w, n, vbits, conv, V, bad, out_keys, out_agg, capacity, n_unique_host, stream);
+}
+
+int glove_cooc_chunk_stanford(const uint64_t *tokens, int64_t n_positions, int64_t n_tokens, int32_t V, int32_t window,
+                           int32_t distance_weighting, void *workspace, size_t workspace_bytes, uint64_t *out_keys,
+                           int64_t *out_agg, int64_t capacity, int64_t *n_unique_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(tokens && workspace && out_keys && out_agg && n_unique_host, "glove_cooc_chunk_stanford: null pointer");
+    GLOVE_REQUIRE(n_positions > 0 && n_tokens >= n_positions && V > 0 && window >= 1 && window <= kStanfordMaxWindow,
+                  "glove_cooc_chunk_stanford: bad sizes (window must be 1..%d)", kStanfordMaxWindow);
+    const int64_t n = n_positions * window;
+    GLOVE_REQUIRE(n < (1ll << 31), "glove_cooc_chunk_stanford: more than 2^31 pairs in one chunk");
+    const int vbits = vbits_of((int64_t)V + 1);
+    GLOVE_REQUIRE(2 * vbits <= 62, "glove_cooc_chunk_stanford: vocabulary too large");
+    const CoocWs w = cooc_ws_view(workspace, n);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "glove_cooc_chunk_stanford: workspace %zu < required %zu", workspace_bytes, w.bytes);
+    int32_t *bad = (int32_t *)w.flags;
+    GLOVE_CHECK_CUDA(cudaMemsetAsync(bad, 0, sizeof(int32_t), stream));
+    emit_line_pairs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tokens, n_positions, n_tokens, window, vbits, V,
+                                                                             w.keys[0], w.kk[0], bad);
+    GLOVE_CHECK_LAUNCH();
+    KToAgg16 conv;
+    const long long unit = lcm_upto(window);
+    for (int k = 0; k < 16; ++k) conv.w[k] = k >= window ? 0 : distance_weighting ? unit / (k + 1) : 1;
+    return reduce_chunk_pairs("glove_cooc_chunk_stanford", w, n, vbits, conv, V, bad, out_keys, out_agg, capacity, n_unique_host,
+                              stream);
 }
 
 int glove_cooc_merge(const uint64_t *keys_a, const int64_t *agg_a, int64_t n_a, const uint64_t *keys_b, const int64_t *agg_b,
@@ -400,37 +506,23 @@ int glove_cooc_route(const uint64_t *keys, const int64_t *agg, int64_t n, int32_
                   "glove_cooc_route: bad sizes (part_bits must be 0..%d)", kCoocMaxPartBits);
     GLOVE_REQUIRE(2 * n < (1ll << 31), "glove_cooc_route: more than 2^30 entries");
     GLOVE_REQUIRE(capacity >= 2 * n, "glove_cooc_route: capacity %lld < 2n = %lld", (long long)capacity, (long long)(2 * n));
-    const int vbits = vbits_of((int64_t)V + 1);
-    const int64_t n2 = 2 * n;
-    const RouteWs w = route_ws_view(workspace, n2, part_bits);
-    if (workspace_bytes < w.bytes)
-        return set_error(GLOVE_EWORKSPACE, "glove_cooc_route: workspace %zu < required %zu", workspace_bytes, w.bytes);
-    const unsigned g = (unsigned)((n2 + 255) / 256);
-    route_parts_kernel<<<g, 256, 0, stream>>>(keys, n, vbits, order_key, part_bits, w.part[0], w.idx[0]);
-    GLOVE_CHECK_LAUNCH();
-    const uint32_t *order = w.idx[0];
-    const int P = 1 << part_bits;
-    if (part_bits) {
-        size_t tb = w.cub_bytes;
-        GLOVE_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(w.cub_temp, tb, w.part[0], w.part[1], w.idx[0], w.idx[1], (int)n2, 0,
-                                                         part_bits, stream));
-        tb = w.cub_bytes;
-        GLOVE_CHECK_CUDA(cub::DeviceHistogram::HistogramEven(w.cub_temp, tb, w.part[1], w.hist, P + 1, 0u, (uint32_t)P, (int)n2,
-                                                             stream));
-        order = w.idx[1];
-    }
-    route_scatter_kernel<<<g, 256, 0, stream>>>(keys, (const Agg *)agg, n, vbits, order, out_keys, (Agg *)out_agg);
-    GLOVE_CHECK_LAUNCH();
-    if (part_bits) {
-        int hist[1 << kCoocMaxPartBits];
-        GLOVE_CHECK_CUDA(cudaMemcpyAsync(hist, w.hist, sizeof(int) * P, cudaMemcpyDeviceToHost, stream));
-        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
-        for (int p = 0; p < P; ++p) part_count_host[p] = hist[p];
-    } else {
-        GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
-        part_count_host[0] = n2;
-    }
-    return GLOVE_OK;
+    return route_entries("glove_cooc_route", keys, agg, n, 2, V, order_key, part_bits, workspace, workspace_bytes, out_keys,
+                         out_agg, part_count_host, stream);
+}
+
+int glove_cooc_route_stanford(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, uint64_t order_key, int32_t part_bits,
+                           int32_t symmetric, void *workspace, size_t workspace_bytes, uint64_t *out_keys, int64_t *out_agg,
+                           int64_t capacity, int64_t *part_count_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(keys && agg && workspace && out_keys && out_agg && part_count_host, "glove_cooc_route_stanford: null pointer");
+    GLOVE_REQUIRE(n > 0 && V > 0 && part_bits >= 0 && part_bits <= kCoocMaxPartBits,
+                  "glove_cooc_route_stanford: bad sizes (part_bits must be 0..%d)", kCoocMaxPartBits);
+    GLOVE_REQUIRE(2 * n < (1ll << 31), "glove_cooc_route_stanford: more than 2^30 entries");
+    const int n_orient = symmetric ? 2 : 1;
+    GLOVE_REQUIRE(capacity >= n_orient * n, "glove_cooc_route_stanford: capacity %lld < %lld", (long long)capacity,
+                  (long long)(n_orient * n));
+    return route_entries("glove_cooc_route_stanford", keys, agg, n, n_orient, V, order_key, part_bits, workspace, workspace_bytes,
+                         out_keys, out_agg, part_count_host, stream);
 }
 
 int glove_cooc_finish_sorted(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t context, int64_t count_min,
@@ -449,6 +541,26 @@ int glove_cooc_finish_sorted(const uint64_t *keys, const int64_t *agg, int64_t n
     return finish_records("glove_cooc_finish_sorted", keys, (const Agg *)agg, n, w, vbits, context, count_min, vocab_count,
                           total_tokens, order_key, row, col, count, value, neg_weight, glove_weight, glove_value, capacity,
                           n_out_host, stream);
+}
+
+int glove_cooc_finish_stanford(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t window,
+                            int32_t distance_weighting, const int64_t *vocab_count, int64_t total_tokens, uint64_t order_key,
+                            void *workspace, size_t workspace_bytes, int32_t *row, int32_t *col, int64_t *count, double *value,
+                            double *neg_weight, double *glove_weight, double *glove_value, int64_t capacity,
+                            int64_t *n_out_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(keys && agg && vocab_count && workspace && n_out_host && n > 0, "glove_cooc_finish_stanford: bad arguments");
+    GLOVE_REQUIRE(window >= 1 && window <= kStanfordMaxWindow && total_tokens > 0 && V > 0,
+                  "glove_cooc_finish_stanford: bad sizes (window must be 1..%d)", kStanfordMaxWindow);
+    GLOVE_REQUIRE(n < (1ll << 31), "glove_cooc_finish_stanford: more than 2^31 entries");
+    const int vbits = vbits_of((int64_t)V + 1);
+    const CoocWs w = cooc_ws_view(workspace, n);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "glove_cooc_finish_stanford: workspace %zu < required %zu", workspace_bytes, w.bytes);
+    // every pair is a record (count_min 1); value = numer / lcm(1..window), or count with unit weights
+    return finish_records("glove_cooc_finish_stanford", keys, (const Agg *)agg, n, w, vbits, distance_weighting ? window : 1, 1,
+                          vocab_count, total_tokens, order_key, row, col, count, value, neg_weight, glove_weight, glove_value,
+                          capacity, n_out_host, stream);
 }
 
 }  // extern "C"

@@ -230,7 +230,8 @@ struct FieldBytes {
 };
 
 __device__ int32_t lookup_token(const Bytes &text, const Field &f, const int32_t *__restrict__ table,
-                                int64_t slots, const uint8_t *__restrict__ vb, const int64_t *__restrict__ voff) {
+                                int64_t slots, const uint8_t *__restrict__ vb, const int64_t *__restrict__ voff,
+                                int32_t missing = 0) {
     uint64_t h = kFnvSeed;
     int len = 0;
     {
@@ -241,7 +242,7 @@ __device__ int32_t lookup_token(const Bytes &text, const Field &f, const int32_t
     uint32_t s = slot_of(h, slots);
     for (;;) {
         const int32_t v = table[s];
-        if (v < 0) return 0;                       // StaticHashTable default_value = 0
+        if (v < 0) return missing;                 // StaticHashTable default_value = 0
         const int64_t o0 = voff[v];
         if (voff[v + 1] - 1 - o0 == len) {
             FieldBytes it = {text, f.b, f.e, f.esc != 0};
@@ -430,6 +431,7 @@ __global__ void __launch_bounds__(256) token_runs_kernel(const uint32_t *__restr
     first_len[r] = lens[head];
     count[r] = run_len[r];
 }
+template <int32_t kMissing>
 __global__ void __launch_bounds__(256) token_lookup_kernel(const uint8_t *__restrict__ text, const int64_t *__restrict__ starts,
                                                            const int32_t *__restrict__ lens, int64_t n,
                                                            const int32_t *__restrict__ table, int64_t slots,
@@ -439,7 +441,53 @@ __global__ void __launch_bounds__(256) token_lookup_kernel(const uint8_t *__rest
     if (i >= n) return;
     const Bytes t = {text + starts[i]};
     const Field f = {0, lens[i], 0};
-    ids[i] = lookup_token(t, f, table, slots, vb, voff);
+    ids[i] = lookup_token(t, f, table, slots, vb, voff, kMissing);
+}
+
+// ---- Stanford GloVe's token stream (vocab_count / cooccur semantics, corpus.py scheme "stanford") ----------------------
+// Bytes that Stanford's get_word glues into tokens (it splits on ' ', '\t', '\n' only and drops every '\r') but that this
+// project's vocabulary readers would split: \v, \f, 0x1c-0x1f, and a \r that is not directly before a \n.  With these
+// refused, the token boundaries of Stanford's tokenizer are those of glove_tokens_scan.  next_byte: the byte after the
+// chunk (-1 at the end of the file).  The lowest offending offset wins.
+__device__ __forceinline__ bool refused_byte(uint8_t b, int32_t next) {
+    return b == 0x0b || b == 0x0c || (b >= 0x1c && b <= 0x1f) || (b == 0x0d && next != 0x0a);
+}
+__global__ void __launch_bounds__(256) text_refused_kernel(const uint8_t *__restrict__ text, int64_t nbytes, int32_t next_byte,
+                                                           unsigned long long *first) {
+    const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 16;
+    if (i0 >= nbytes) return;
+    alignas(16) uint8_t b[16];
+    if (i0 + 16 <= nbytes) *(uint4 *)b = __ldg((const uint4 *)(text + i0));
+    else
+        for (int k = 0; k < 16; ++k) b[k] = i0 + k < nbytes ? text[i0 + k] : (uint8_t)' ';
+    const int32_t after = i0 + 16 < nbytes ? (int32_t)text[i0 + 16] : i0 + 16 == nbytes ? next_byte : -1;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+        if (refused_byte(b[k], k < 15 ? (int32_t)b[k + 1] : after)) {
+            atomicMin(first, (unsigned long long)(i0 + k));
+            return;
+        }
+    }
+}
+// brk[i] = 1 when a '\n' lies between token i - 1 and token i (token 0: between text_begin and its start, or
+// newline_before, a '\n' after the last token of the previous chunk)
+__global__ void __launch_bounds__(256) token_breaks_kernel(const uint8_t *__restrict__ text, int64_t text_begin,
+                                                           const int64_t *__restrict__ starts, const int32_t *__restrict__ lens,
+                                                           int64_t n, int32_t newline_before, uint32_t *brk) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t lo = i ? starts[i - 1] + lens[i - 1] : text_begin;
+    bool nl = i == 0 && newline_before;
+    for (int64_t e = starts[i] - 1; !nl && e >= lo; --e) nl = text[e] == '\n';
+    brk[i] = nl;
+}
+// in-vocabulary tokens as (segment << 32) | id, segment = segment_base + number of line breaks up to the token
+__global__ void __launch_bounds__(256) token_pack_kernel(const int32_t *__restrict__ ids, const uint32_t *__restrict__ seg,
+                                                         int64_t n, uint32_t segment_base, uint64_t *packed, uint8_t *keep) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    packed[i] = ((uint64_t)(segment_base + seg[i]) << 32) | (uint32_t)ids[i];
+    keep[i] = ids[i] >= 0;
 }
 
 struct TokWs {
@@ -476,6 +524,36 @@ static TokWs tok_ws_view(void *base, int64_t nbytes, int64_t n_tokens) {
     if (c > w.cub_bytes) w.cub_bytes = c;
     if (d > w.cub_bytes) w.cub_bytes = d;
     if (e > w.cub_bytes) w.cub_bytes = e;
+    w.cub_temp = take(w.cub_bytes);
+    w.bytes = off;
+    return w;
+}
+
+struct StreamWs {
+    int32_t *ids;
+    uint32_t *brk, *seg;
+    uint64_t *packed;
+    uint8_t *keep;
+    long long *n_out;
+    void *cub_temp;
+    size_t cub_bytes, bytes;
+};
+static StreamWs stream_ws_view(void *base, int64_t n) {
+    StreamWs w;
+    char *p = (char *)base;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char *r = p ? p + off : nullptr; off += align_up(bytes); return r; };
+    w.ids = (int32_t *)take(4 * n);
+    w.brk = (uint32_t *)take(4 * n);
+    w.seg = (uint32_t *)take(4 * n);
+    w.packed = (uint64_t *)take(8 * n);
+    w.keep = (uint8_t *)take(n);
+    w.n_out = (long long *)take(8);
+    size_t a = 0, b = 0;
+    cub::DeviceScan::InclusiveSum(nullptr, a, (uint32_t *)nullptr, (uint32_t *)nullptr, (int)n);
+    cub::DeviceSelect::Flagged(nullptr, b, (uint64_t *)nullptr, (uint8_t *)nullptr, (uint64_t *)nullptr, (long long *)nullptr,
+                               (int)n);
+    w.cub_bytes = a > b ? a : b;
     w.cub_temp = take(w.cub_bytes);
     w.bytes = off;
     return w;
@@ -670,9 +748,66 @@ int glove_tokens_lookup(const uint8_t *text, const int64_t *starts, const int32_
                         int32_t *ids, void *stream) {
     GLOVE_REQUIRE(text && starts && lens && vocab_table && vocab_bytes && vocab_off && ids && n_tokens > 0 && vocab_slots > 0,
                   "glove_tokens_lookup: bad arguments");
-    token_lookup_kernel<<<(unsigned)((n_tokens + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+    token_lookup_kernel<0><<<(unsigned)((n_tokens + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         text, starts, lens, n_tokens, vocab_table, vocab_slots, vocab_bytes, vocab_off, ids);
     GLOVE_CHECK_LAUNCH();
+    return GLOVE_OK;
+}
+
+int glove_text_refused(const uint8_t *text, int64_t nbytes, int32_t next_byte, uint64_t *scratch, int64_t *first_host,
+                       void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(text && scratch && first_host, "glove_text_refused: null pointer");
+    GLOVE_REQUIRE(nbytes > 0 && nbytes < (1ll << 40) && next_byte >= -1 && next_byte <= 255, "glove_text_refused: bad sizes");
+    GLOVE_REQUIRE(((uintptr_t)text & 15) == 0, "glove_text_refused: text must be 16-byte aligned");
+    GLOVE_CHECK_CUDA(cudaMemsetAsync(scratch, 0xff, 8, stream));
+    const int64_t threads = (nbytes + 15) / 16;
+    text_refused_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(text, nbytes, next_byte,
+                                                                              (unsigned long long *)scratch);
+    GLOVE_CHECK_LAUNCH();
+    uint64_t first = 0;
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(&first, scratch, 8, cudaMemcpyDeviceToHost, stream));
+    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    *first_host = first == ~0ull ? -1 : (int64_t)first;
+    return GLOVE_OK;
+}
+
+size_t glove_tokens_stream_workspace_bytes(int64_t n_tokens) { return stream_ws_view(nullptr, n_tokens < 1 ? 1 : n_tokens).bytes; }
+
+int glove_tokens_stream(const uint8_t *text, int64_t text_begin, const int64_t *starts, const int32_t *lens, int64_t n_tokens,
+                        int32_t newline_before, uint32_t segment_base, const int32_t *vocab_table, int64_t vocab_slots,
+                        const uint8_t *vocab_bytes, const int64_t *vocab_off, void *workspace, size_t workspace_bytes,
+                        uint64_t *out, int64_t capacity, int64_t *n_out_host, uint32_t *last_segment_host, void *stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    GLOVE_REQUIRE(text && starts && lens && vocab_table && vocab_bytes && vocab_off && workspace && out && n_out_host &&
+                      last_segment_host,
+                  "glove_tokens_stream: null pointer");
+    GLOVE_REQUIRE(n_tokens > 0 && n_tokens < (1ll << 31) && text_begin >= 0 && vocab_slots > 0,
+                  "glove_tokens_stream: bad sizes");
+    GLOVE_REQUIRE(capacity >= n_tokens, "glove_tokens_stream: capacity %lld < n_tokens %lld", (long long)capacity,
+                  (long long)n_tokens);
+    const StreamWs w = stream_ws_view(workspace, n_tokens);
+    if (workspace_bytes < w.bytes)
+        return set_error(GLOVE_EWORKSPACE, "glove_tokens_stream: workspace %zu < required %zu", workspace_bytes, w.bytes);
+    const unsigned g = (unsigned)((n_tokens + 255) / 256);
+    token_lookup_kernel<-1><<<g, 256, 0, stream>>>(text, starts, lens, n_tokens, vocab_table, vocab_slots, vocab_bytes, vocab_off,
+                                                   w.ids);
+    GLOVE_CHECK_LAUNCH();
+    token_breaks_kernel<<<g, 256, 0, stream>>>(text, text_begin, starts, lens, n_tokens, newline_before, w.brk);
+    GLOVE_CHECK_LAUNCH();
+    size_t tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceScan::InclusiveSum(w.cub_temp, tb, w.brk, w.seg, (int)n_tokens, stream));
+    token_pack_kernel<<<g, 256, 0, stream>>>(w.ids, w.seg, n_tokens, segment_base, w.packed, w.keep);
+    GLOVE_CHECK_LAUNCH();
+    tb = w.cub_bytes;
+    GLOVE_CHECK_CUDA(cub::DeviceSelect::Flagged(w.cub_temp, tb, w.packed, w.keep, out, w.n_out, (int)n_tokens, stream));
+    long long n = 0;
+    uint32_t last = 0;
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(&n, w.n_out, 8, cudaMemcpyDeviceToHost, stream));
+    GLOVE_CHECK_CUDA(cudaMemcpyAsync(&last, w.seg + n_tokens - 1, 4, cudaMemcpyDeviceToHost, stream));
+    GLOVE_CHECK_CUDA(cudaStreamSynchronize(stream));
+    *n_out_host = n;
+    *last_segment_host = segment_base + last;
     return GLOVE_OK;
 }
 

@@ -417,6 +417,22 @@ int glove_tokens_count(const uint8_t *text, int64_t nbytes, const int64_t *start
 int glove_tokens_lookup(const uint8_t *text, const int64_t *starts, const int32_t *lens, int64_t n_tokens,
                         const int32_t *vocab_table, int64_t vocab_slots, const uint8_t *vocab_bytes, const int64_t *vocab_off,
                         int32_t *ids, void *stream);
+/* Stanford GloVe's token stream (corpus.py, scheme "stanford").  glove_text_refused: the lowest offset in text[0, nbytes)
+ * of a byte Stanford's tokenizer would glue into a token but glove_tokens_scan splits on (\v, \f, 0x1c-0x1f, a \r not
+ * directly before \n; next_byte = the byte after the chunk, -1 at the end of the file), or -1.  scratch: 8 device
+ * bytes; text 16-byte aligned.  Synchronises.
+ * glove_tokens_stream: the in-vocabulary tokens among the n_tokens of glove_tokens_scan, in text order, as
+ * out[j] = (segment << 32) | id (id = line of the vocab table, out-of-vocabulary tokens removed; segment =
+ * segment_base + the number of '\n' bytes before the token, counted from text_begin, plus 1 when newline_before; uint32,
+ * wrapping).  *last_segment_host: the segment of token n_tokens - 1, kept or not (the segment_base of the next chunk).
+ * capacity >= n_tokens.  Workspace: glove_tokens_stream_workspace_bytes(n_tokens).  Synchronises. */
+int glove_text_refused(const uint8_t *text, int64_t nbytes, int32_t next_byte, uint64_t *scratch, int64_t *first_host,
+                       void *stream);
+size_t glove_tokens_stream_workspace_bytes(int64_t n_tokens);
+int glove_tokens_stream(const uint8_t *text, int64_t text_begin, const int64_t *starts, const int32_t *lens, int64_t n_tokens,
+                        int32_t newline_before, uint32_t segment_base, const int32_t *vocab_table, int64_t vocab_slots,
+                        const uint8_t *vocab_bytes, const int64_t *vocab_off, void *workspace, size_t workspace_bytes,
+                        uint64_t *out, int64_t capacity, int64_t *n_out_host, uint32_t *last_segment_host, void *stream);
 
 /* ---- PREPROCESS: token-id stream -> symmetric co-occurrence table with the GloVe columns (SURVEY 8 f.4) ------------
  * create_interaction_dataframe + create_glove_dataframe of the reference preprocessor [ref src/data/text8.py:84-139].
@@ -453,6 +469,23 @@ size_t glove_cooc_route_workspace_bytes(int64_t n, int32_t part_bits);
 int glove_cooc_route(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, uint64_t order_key, int32_t part_bits,
                      void *workspace, size_t workspace_bytes, uint64_t *out_keys, int64_t *out_agg, int64_t capacity,
                      int64_t *part_count_host, void *stream);
+/* The Stanford GloVe scheme (cooccur's counting rules).  glove_cooc_chunk_stanford: tokens as from glove_tokens_stream;
+ * for positions p < n_positions and k = 1..window (1..15) with p + k < n_tokens and both on one segment, the pair
+ * (id[p], id[p + k]), self pairs included, with weight lcm(1..window) / k (distance_weighting) or 1; reduced as
+ * glove_cooc_chunk.  glove_cooc_route_stanford: glove_cooc_route with both orientations (symmetric) or only (a, b);
+ * capacity >= 2n or n.  glove_cooc_finish_stanford: glove_cooc_finish_sorted with count_min 1 and value = numer /
+ * lcm(1..window) (distance_weighting) or count.  Same workspaces and synchronisation as their reference counterparts. */
+int glove_cooc_chunk_stanford(const uint64_t *tokens, int64_t n_positions, int64_t n_tokens, int32_t V, int32_t window,
+                              int32_t distance_weighting, void *workspace, size_t workspace_bytes, uint64_t *out_keys,
+                              int64_t *out_agg, int64_t capacity, int64_t *n_unique_host, void *stream);
+int glove_cooc_route_stanford(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, uint64_t order_key,
+                              int32_t part_bits, int32_t symmetric, void *workspace, size_t workspace_bytes, uint64_t *out_keys,
+                              int64_t *out_agg, int64_t capacity, int64_t *part_count_host, void *stream);
+int glove_cooc_finish_stanford(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t window,
+                               int32_t distance_weighting, const int64_t *vocab_count, int64_t total_tokens, uint64_t order_key,
+                               void *workspace, size_t workspace_bytes, int32_t *row, int32_t *col, int64_t *count,
+                               double *value, double *neg_weight, double *glove_weight, double *glove_value, int64_t capacity,
+                               int64_t *n_out_host, void *stream);
 /* glove_cooc_finish for a table that is already symmetric (one partition merged from routed entries): no transpose.
  * Workspace: glove_cooc_workspace_bytes(n). */
 int glove_cooc_finish_sorted(const uint64_t *keys, const int64_t *agg, int64_t n, int32_t V, int32_t context, int64_t count_min,
