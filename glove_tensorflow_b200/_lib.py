@@ -174,6 +174,15 @@ SIGNATURES = {
     "glove_cooc_bin_parse": (ctypes.c_int, [c_void, c_i64, c_i64, c_i64, ctypes.c_double, ctypes.c_double, c_void, c_void,
                                             c_void, c_void, c_void, c_void]),
     "glove_cooc_bin_format": (ctypes.c_int, [c_void, c_void, c_void, c_i64, c_void, c_void]),
+    "glove_sgd_parse": (ctypes.c_int, [c_void, c_i64, c_i64, c_i64, ctypes.c_double, ctypes.c_double, c_void, c_void, c_void,
+                                       c_void]),
+    "glove_sgd_links_workspace_bytes": (c_size, [c_i64]),
+    "glove_sgd_links": (ctypes.c_int, [c_void, c_i64, c_i64, c_void, c_void, c_size, c_void]),
+    "glove_sgd_init": (ctypes.c_int, [c_void, c_i64, c_i32, ctypes.c_uint64, c_void]),
+    "glove_sgd_epoch_workspace_bytes": (c_size, [c_i64]),
+    "glove_sgd_epoch": (ctypes.c_int, [c_void, c_void, c_i64, c_i32, c_void, c_void, c_void, c_i64, ctypes.c_double,
+                                       ctypes.c_double, c_i32, c_void, c_i32, c_void, c_size, c_void, c_void]),
+    "glove_sgd_rows": (ctypes.c_int, [c_void, c_i64, c_i32, c_i32, c_i32, c_void, c_void]),
     "glove_host_staging_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_plan_bytes": (c_size, [c_i32, c_i32]),
     "glove_host_pipe_create": (ctypes.c_int, [ctypes.POINTER(c_void)]),

@@ -27,10 +27,7 @@ __global__ void __launch_bounds__(kCrecThreads) crec_parse_kernel(const int4 *__
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const int4 r = __ldcs(rec + i);
         const double val = __hiloint2double(r.w, r.z);
-        int kind = -1;
-        if (r.x < 1 || r.x > V) kind = GLOVE_CREC_BAD_WORD1;
-        else if (r.y < 1 || r.y > V) kind = GLOVE_CREC_BAD_WORD2;
-        else if (!(val > 0.0 && val <= 1.7976931348623157e308)) kind = GLOVE_CREC_BAD_VALUE;
+        GLOVE_CREC_KIND(kind, r, val, V);
         if (kind >= 0 && bad == ~0ull) bad = (unsigned long long)(first + i) * 4 + kind;   // i ascends: first bad is lowest
         row[i] = r.x - 1;
         col[i] = r.y - 1;

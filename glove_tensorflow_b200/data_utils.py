@@ -309,17 +309,40 @@ def load_cooc_bin(path, vocab_size, x_max=100.0, alpha=0.75, device="cuda:0", ch
     offset."""
     import torch
     from . import _lib
-    lib, check = _lib.lib, _lib.check
-    V = int(vocab_size)
-    if not 1 <= V < (1 << 31):
-        raise ValueError("vocab_size must be 1 .. 2^31-1, got %d" % V)
-    size = os.path.getsize(path)
-    n = size // COOC_RECORD
+    V = _check_vocab_size(vocab_size)
+    n = os.path.getsize(path) // COOC_RECORD
     dev = torch.device(device)
     with torch.cuda.device(dev):
         out = {"row": torch.empty(n, dtype=torch.int32, device=dev), "col": torch.empty(n, dtype=torch.int32, device=dev),
                "glove_value": torch.empty(n, dtype=torch.float32, device=dev),
                "glove_weight": torch.empty(n, dtype=torch.float32, device=dev)}
+
+    def parse(raw, m, first, err, st):
+        _lib.check(_lib.lib.glove_cooc_bin_parse(raw, m, first, V, float(x_max), float(alpha),
+                                                 *[out[c][first:].data_ptr() for c in ("row", "col", "glove_value",
+                                                                                       "glove_weight")],
+                                                 err, st), "glove_cooc_bin_parse")
+
+    stream_cooc_bin(path, V, parse, dev, chunk_bytes)
+    return out
+
+
+def _check_vocab_size(vocab_size):
+    V = int(vocab_size)
+    if not 1 <= V < (1 << 31):
+        raise ValueError("vocab_size must be 1 .. 2^31-1, got %d" % V)
+    return V
+
+
+def stream_cooc_bin(path, V, parse, dev, chunk_bytes=64 << 20):
+    """Streams the whole records of a Stanford co-occurrence file to the device in chunks and calls
+    ``parse(raw_ptr, m, first, error_ptr, stream)`` on each (m records, the first with the 0-based index ``first``), which
+    launches a parser that lowers the error word as glove_cooc_bin_parse does.  Raises on the lowest bad record and on a
+    file cut inside a record."""
+    import torch
+    size = os.path.getsize(path)
+    n = size // COOC_RECORD
+    with torch.cuda.device(dev):
         if n:
             st = torch.cuda.current_stream().cuda_stream
             whole = n * COOC_RECORD
@@ -336,9 +359,7 @@ def load_cooc_bin(path, vocab_size, x_max=100.0, alpha=0.75, device="cuda:0", ch
                     reader.start(k + 1)
                     m, first = nb // COOC_RECORD, k * (chunk // COOC_RECORD)
                     raw[:nb].copy_(pinned[k % len(pinned)][_HEAD:_HEAD + nb], non_blocking=True)
-                    check(lib.glove_cooc_bin_parse(raw.data_ptr(), m, first, V, float(x_max), float(alpha),
-                                                   *[out[c][first:].data_ptr() for c in ("row", "col", "glove_value", "glove_weight")],
-                                                   err.data_ptr(), st), "glove_cooc_bin_parse")
+                    parse(raw.data_ptr(), m, first, err.data_ptr(), st)
                     code = int(err.item()) & 0xFFFFFFFFFFFFFFFF       # synchronises: pinned[k % 2] may be refilled after this
                     if code != 0xFFFFFFFFFFFFFFFF:
                         g = code >> 2
@@ -349,7 +370,6 @@ def load_cooc_bin(path, vocab_size, x_max=100.0, alpha=0.75, device="cuda:0", ch
     if size % COOC_RECORD:
         raise ValueError("%s: record %d (byte %d): the file ends %d bytes into a %d-byte record (truncated file)"
                          % (path, n + 1, n * COOC_RECORD, size % COOC_RECORD, COOC_RECORD))
-    return out
 
 
 def check_ids(row, col, n_vocab, what="COO"):

@@ -542,6 +542,35 @@ int glove_cooc_bin_parse(const void *records, int64_t n, int64_t first_record, i
 int glove_cooc_bin_format(const int32_t *row, const int32_t *col, const double *value, int64_t n, void *records,
                           void *stream);
 
+/* Stanford GloVe's trainer (glove.c with one thread), exact on the GPU (DESIGN.md section 3).  State in glove.c's layout:
+ * W and gradsq are 2V rows of d + 1 doubles (rows 0..V-1 word vectors, V..2V-1 context vectors, last element the bias).
+ * glove_sgd_parse: like glove_cooc_bin_parse (same validation and error word), into the trainer's 24-byte records:
+ * words[2i .. 2i+1] = {word1 - 1, word2 - 1}, lf[2i .. 2i+1] = {log(val), val > x_max ? 1 : pow(val / x_max, alpha)} in
+ * float64 (words 8-byte, lf and records 16-byte aligned).  Asynchronous.
+ * glove_sgd_links: prev[2j] = the last record before j with the same word1, prev[2j+1] the same for word2, -1 if none
+ * (stable radix sort per side).  Asynchronous.
+ * glove_sgd_init: W[i] = (u - 0.5) / d for the 2V(d+1) elements, u = (splitmix64(seed * 0xD1B54A32D192ED03 +
+ * i * 0x9E3779B97F4A7C15) >> 11) * 2^-53.  Asynchronous.
+ * glove_sgd_epoch: one pass over the n records in file order, exactly glove.c's recurrence (1 <= d <= 512).  done[n]
+ * starts at zero and receives `epoch`, which must grow from call to call (1, 2, ...) on the same done array.  grid = 0:
+ * every CTA that fits, else that many CTAs (any value gives the same bits).  *cost (device) receives the summed record
+ * costs / n.  Synchronises; a dependency link that does not point backwards fails with GLOVE_EINVAL, a wait of about a
+ * second with GLOVE_ECUDA.
+ * glove_sgd_rows: out (float32, V + unk rows) = per word the row of a vectors file: model 0 = W row and W~ row with
+ * biases (2d + 2 values), 1 = W (d values), 2 = W + W~ summed in float64 (d values); unk = 1 adds glove.c's <unk> row
+ * from the per-element mean (each term divided by m, then summed) of the last m = min(100, V) rows.  Asynchronous. */
+int glove_sgd_parse(const void *records, int64_t n, int64_t first_record, int64_t V, double x_max, double alpha,
+                    int32_t *words, double *lf, unsigned long long *error, void *stream);
+size_t glove_sgd_links_workspace_bytes(int64_t n);
+int glove_sgd_links(const int32_t *words, int64_t n, int64_t V, int32_t *prev, void *workspace, size_t workspace_bytes,
+                    void *stream);
+int glove_sgd_init(double *W, int64_t V, int32_t d, uint64_t seed, void *stream);
+size_t glove_sgd_epoch_workspace_bytes(int64_t n);
+int glove_sgd_epoch(double *W, double *gradsq, int64_t V, int32_t d, const int32_t *words, const double *lf,
+                    const int32_t *prev, int64_t n, double eta, double grad_clip, int32_t epoch, int32_t *done,
+                    int32_t grid, void *workspace, size_t workspace_bytes, double *cost, void *stream);
+int glove_sgd_rows(const double *W, int64_t V, int32_t d, int32_t model, int32_t unk, float *out, void *stream);
+
 /* ---- HOST-buffer boundary (end to end): what a non-torch caller of the reference's training path would bind ----- */
 /* Runs K TRAIN steps (K a multiple of args->plan_K, at most 4096) on K*B explicit triples held in HOST memory (pinned
  * recommended) and copies the K losses back to host_losses.  Internally a pipeline over the chunks of plan_K steps:
