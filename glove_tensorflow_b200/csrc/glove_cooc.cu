@@ -183,6 +183,29 @@ __global__ void __launch_bounds__(256) order_keys_kernel(const uint64_t *__restr
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) hashed[i] = mix64(keys[sel[i]] + salt * 0x9e3779b97f4a7c15ull);
 }
+// numer / unit rounded once to the nearest double, ties to even, for 0 <= numer < 2^63 and 1 <= unit <= 2^20 (unit is
+// lcm(1..window) <= 360,360).  Below 2^53 both operands convert exactly and IEEE division rounds once.  Above, q = numer
+// / unit has 34..63 bits: with s = bits(q) - 53 > 0 the dropped bits of q and r / unit decide the rounding against half
+// of 2^s (low * unit + r against unit * 2^(s-1), both <= 2^30); with s <= 0 the -s <= 19 fraction bits of r / unit are
+// appended to q and the remainder decides it.  m <= 2^53 and 2^s are exact, so the result is the one rounding.
+__device__ __forceinline__ double div_rn_i64(long long numer, long long unit) {
+    if (numer < (1ll << 53)) return (double)numer / (double)unit;
+    const unsigned long long u = unit, q = (unsigned long long)numer / u, r = (unsigned long long)numer % u;
+    const int s = 64 - __clzll(q) - 53;
+    unsigned long long m, t, h;
+    if (s > 0) {
+        m = q >> s;
+        t = (q & ((1ull << s) - 1)) * u + r;
+        h = u << (s - 1);
+    } else {
+        t = r << -s;
+        m = (q << -s) + t / u;
+        t = 2 * (t % u);
+        h = u;
+    }
+    return ldexp((double)(m + (t > h || (t == h && (m & 1)))), s);
+}
+
 __global__ void __launch_bounds__(256) columns_kernel(const uint64_t *__restrict__ keys, const Agg *__restrict__ agg,
                                                       const uint32_t *__restrict__ order, int64_t n, int vbits, double inv_unit,
                                                       long long unit, const long long *__restrict__ vocab_count,
@@ -195,7 +218,7 @@ __global__ void __launch_bounds__(256) columns_kernel(const uint64_t *__restrict
     const uint64_t k = keys[j];
     const int32_t a = (int32_t)(k >> vbits), b = (int32_t)(k & ((1ull << vbits) - 1));
     const Agg g = agg[j];
-    const double v = (double)g.numer / (double)unit;          // exact integer / small integer: one rounding
+    const double v = div_rn_i64(g.numer, unit);               // exact integer / small integer: one rounding
     row[i] = a;
     col[i] = b;
     count[i] = g.count;

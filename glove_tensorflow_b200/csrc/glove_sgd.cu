@@ -132,12 +132,14 @@ template <int K>
 __global__ void __launch_bounds__(kSgdThreads) sgd_epoch_kernel(const SgdEpoch p) {
     const int lane = threadIdx.x & 31, d = p.d;
     const int64_t ld = d + 1;
-    int next = 0;
-    if (lane == 0) next = atomicAdd(p.ctrl, 1);
+    // Tickets are unsigned: a warp claims tickets until one is >= n, so the largest is n - 1 + (warps in the grid), below
+    // 2^32 for n < 2^31 and grid * 8 < 2^31 warps.  A signed ticket would wrap to -2^31 past n = 2^31 - 1 and pass the test.
+    unsigned next = 0;
+    if (lane == 0) next = atomicAdd((unsigned *)p.ctrl, 1u);
     next = __shfl_sync(0xffffffffu, next, 0);
-    while (next < p.n) {
-        const int j = next;
-        if (lane == 0) next = atomicAdd(p.ctrl, 1);   // claim the next record now: the atomic overlaps this one
+    while (next < (unsigned)p.n) {
+        const int j = (int)next;
+        if (lane == 0) next = atomicAdd((unsigned *)p.ctrl, 1u);   // claim the next record now: the atomic overlaps this one
         const int2 w = p.words[j];
         const double2 lf = p.lf[j];
         const int2 pv = p.prev[j];
@@ -345,7 +347,7 @@ int glove_sgd_epoch(double *W, double *gradsq, int64_t V, int32_t d, const int32
     GLOVE_REQUIRE(V >= 1 && V < (1ll << 31), "glove_sgd_epoch: V must be 1 .. 2^31-1");
     GLOVE_REQUIRE(d >= 1 && d <= 32 * kSgdMaxK, "glove_sgd_epoch: d must be 1 .. %d", 32 * kSgdMaxK);
     GLOVE_REQUIRE(n >= 1 && n < (1ll << 31), "glove_sgd_epoch: n must be 1 .. 2^31-1");
-    GLOVE_REQUIRE(epoch >= 1 && grid >= 0, "glove_sgd_epoch: epoch must be >= 1 and grid >= 0");
+    GLOVE_REQUIRE(epoch >= 1 && grid >= 0 && grid < (1 << 28), "glove_sgd_epoch: epoch must be >= 1 and grid 0 .. 2^28 - 1");
     GLOVE_REQUIRE(eta == eta && grad_clip == grad_clip, "glove_sgd_epoch: eta and grad_clip must not be NaN");
     GLOVE_REQUIRE(((uintptr_t)lf & 15) == 0 && ((uintptr_t)words & 7) == 0 && ((uintptr_t)prev & 7) == 0,
                   "glove_sgd_epoch: lf must be 16-byte aligned, words and prev 8-byte aligned");

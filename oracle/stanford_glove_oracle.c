@@ -22,9 +22,13 @@ static double butterfly(double *v) {
 static double check_nan(double v) { return (isnan(v) || isinf(v)) ? 0.0 : v; }
 
 /* One epoch over n records: W, G are 2V rows of d + 1 doubles; words[2j], words[2j+1] = word1 - 1, word2 - 1;
- * lf[2j], lf[2j+1] = log(val), f.  cost[j] receives the record's cost (0 for a skipped record).  Returns 0. */
+ * lf[2j], lf[2j+1] = log(val), f.  cost[j] receives the record's cost (0 for a skipped record).  hits (may be NULL)
+ * accumulates how often each branch was taken: [0] skipped records, [1] clipped products (fmin / fmax changed
+ * fdiff * W[.][b]), [2] records whose update sums were not finite (vectors kept), [3] bias steps that check_nan zeroed.
+ * Returns 0. */
 int sg_oracle_epoch(int64_t V, int32_t d, double *W, double *G, const int32_t *words, const double *lf, int64_t n,
-                    double eta, double clip, int32_t order, double *cost) {
+                    double eta, double clip, int32_t order, double *cost, int64_t *hits) {
+    int64_t h[4] = {0, 0, 0, 0};
     const int64_t ld = d + 1;
     double *u1 = malloc(sizeof(double) * d), *u2 = malloc(sizeof(double) * d);
     if (!u1 || !u2) return -1;
@@ -42,12 +46,14 @@ int sg_oracle_epoch(int64_t V, int32_t d, double *W, double *G, const int32_t *w
         diff = diff + ((wa[d] + wc[d]) - lf[2 * j]);
         double fdiff = lf[2 * j + 1] * diff;
         cost[j] = 0.0;
-        if (isnan(diff) || isnan(fdiff) || isinf(diff) || isinf(fdiff)) continue;
+        if (isnan(diff) || isnan(fdiff) || isinf(diff) || isinf(fdiff)) { ++h[0]; continue; }
         cost[j] = (0.5 * fdiff) * diff;
         double s1[32] = {0}, s2[32] = {0};
         for (int b = 0; b < d; ++b) {
-            const double t1 = fmin(fmax(fdiff * wc[b], -clip), clip) * eta;
-            const double t2 = fmin(fmax(fdiff * wa[b], -clip), clip) * eta;
+            const double p1 = fdiff * wc[b], p2 = fdiff * wa[b], c1 = fmin(fmax(p1, -clip), clip),
+                         c2 = fmin(fmax(p2, -clip), clip);
+            h[1] += (c1 != p1) + (c2 != p2);
+            const double t1 = c1 * eta, t2 = c2 * eta;
             u1[b] = t1 / sqrt(ga[b]);
             u2[b] = t2 / sqrt(gc[b]);
             const int l = order == 0 ? 0 : (b & 31);
@@ -62,15 +68,21 @@ int sg_oracle_epoch(int64_t V, int32_t d, double *W, double *G, const int32_t *w
                 wa[b] -= u1[b];
                 wc[b] -= u2[b];
             }
+        } else {
+            ++h[2];
         }
-        wa[d] -= check_nan(fdiff / sqrt(ga[d]));
-        wc[d] -= check_nan(fdiff / sqrt(gc[d]));
+        const double ba = fdiff / sqrt(ga[d]), bc = fdiff / sqrt(gc[d]);
+        h[3] += (check_nan(ba) != ba) + (check_nan(bc) != bc);
+        wa[d] -= check_nan(ba);
+        wc[d] -= check_nan(bc);
         fdiff *= fdiff;
         ga[d] += fdiff;
         gc[d] += fdiff;
     }
     free(u1);
     free(u2);
+    if (hits)
+        for (int k = 0; k < 4; ++k) hits[k] += h[k];
     return 0;
 }
 

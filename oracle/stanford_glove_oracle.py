@@ -90,17 +90,21 @@ def init_params(V, d, seed):
     return ((u - 0.5) / d).reshape(2 * V, d + 1)
 
 
-def epoch(W, G, words, lf, eta=0.05, clip=100.0, order=1):
-    """One epoch in place on W, G (C-contiguous float64).  Returns the per-record costs (0 for a skipped record)."""
+def epoch(W, G, words, lf, eta=0.05, clip=100.0, order=1, hits=None):
+    """One epoch in place on W, G (C-contiguous float64).  Returns the per-record costs (0 for a skipped record).
+    ``hits`` (int64 [4], optional) accumulates the branch counts: skipped records, clipped products, records whose
+    update sums were not finite, bias steps zeroed by check_nan."""
     assert W.dtype == G.dtype == np.float64 and W.flags.c_contiguous and G.flags.c_contiguous and W.shape == G.shape
     V, d = W.shape[0] // 2, W.shape[1] - 1
     words = np.ascontiguousarray(words, np.int32)
     lf = np.ascontiguousarray(lf, np.float64)
     cost = np.zeros(len(words), np.float64)
+    if hits is not None:
+        assert hits.dtype == np.int64 and hits.shape == (4,) and hits.flags.c_contiguous
     p = lambda a: a.ctypes.data_as(ctypes.c_void_p)
     rc = lib().sg_oracle_epoch(ctypes.c_int64(V), ctypes.c_int32(d), p(W), p(G), p(words), p(lf),
                                ctypes.c_int64(len(words)), ctypes.c_double(eta), ctypes.c_double(clip),
-                               ctypes.c_int32(order), p(cost))
+                               ctypes.c_int32(order), p(cost), None if hits is None else p(hits))
     assert rc == 0
     return cost
 

@@ -267,7 +267,7 @@ def test_sgd_entries_refuse_bad_arguments_without_a_gpu():
     assert epoch(a0=None) == E and epoch(a11=None) == E and epoch(a15=None) == E
     assert epoch(a2=0) == E and epoch(a3=0) == E and epoch(a3=513) == E and epoch(a7=0) == E and epoch(a7=1 << 31) == E
     assert epoch(a8=float("nan")) == E and epoch(a9=float("nan")) == E
-    assert epoch(a10=0) == E and epoch(a12=-1) == E and epoch(a14=es - 1) == E
+    assert epoch(a10=0) == E and epoch(a12=-1) == E and epoch(a12=1 << 28) == E and epoch(a14=es - 1) == E
     assert epoch(a5=ctypes.c_void_p((1 << 20) + 8)) == E and epoch(a4=ctypes.c_void_p((1 << 20) + 4)) == E
     assert lib.glove_sgd_rows(None, 10, 4, 2, 1, f, None) == E
     assert lib.glove_sgd_rows(f, 10, 4, 3, 1, f, None) == E

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import stanford_glove_oracle as sgo
+from test_stanford_edges_gpu import assert_bits
 
 pytestmark = pytest.mark.gpu
 
@@ -91,16 +92,16 @@ def test_bit_identical_to_the_kernel_order_oracle(tmp_path, kind, d):
     V, n = {"serial": (3000, 20_000), "free": (40_000, 40_000), "zipf": (50_000, 1_000_000)}[kind]
     path = write_bin(tmp_path / "c.bin", *make_table(kind, V, n, d))
     sg = StanfordGlove(path, V, d, seed=7)
-    np.testing.assert_array_equal(sg.W.cpu().numpy(), sgo.init_params(V, d, 7))
+    assert_bits(sg.W.cpu().numpy(), sgo.init_params(V, d, 7), "init")
     W1, G1, c1 = _oracle_run(sg, 1)
     got1 = sg.epoch()
-    np.testing.assert_array_equal(sg.W.cpu().numpy(), W1)
-    np.testing.assert_array_equal(sg.gradsq.cpu().numpy(), G1)
+    assert_bits(sg.W.cpu().numpy(), W1, "W1")
+    assert_bits(sg.gradsq.cpu().numpy(), G1, "G1")
     assert got1 == c1[0]
     W3, G3, c3 = _oracle_run(sg, 3)
     got = [got1, sg.epoch(), sg.epoch()]
-    np.testing.assert_array_equal(sg.W.cpu().numpy(), W3)
-    np.testing.assert_array_equal(sg.gradsq.cpu().numpy(), G3)
+    assert_bits(sg.W.cpu().numpy(), W3, "W3")
+    assert_bits(sg.gradsq.cpu().numpy(), G3, "G3")
     assert got == c3
 
 
@@ -114,8 +115,8 @@ def test_same_bits_for_one_cta_full_grid_and_reruns(tmp_path):
         costs = [sg.epoch(grid=grid) for _ in range(2)]
         runs.append((sg.W.cpu().numpy(), sg.gradsq.cpu().numpy(), costs))
     for W, G, c in runs[1:]:
-        np.testing.assert_array_equal(W, runs[0][0])
-        np.testing.assert_array_equal(G, runs[0][1])
+        assert_bits(W, runs[0][0], "W")
+        assert_bits(G, runs[0][1], "gradsq")
         assert c == runs[0][2]
 
 
@@ -142,7 +143,7 @@ def test_resume_is_exact(tmp_path):
     assert words == ["w%d" % i for i in range(V)] + ["<unk>"]
     from glove_tensorflow_b200.vectors import read_vectors
     _, rows = read_vectors(str(tmp_path / "full.txt"))
-    np.testing.assert_array_equal(rows.cpu().numpy(), sgo.rows(W, 2))
+    assert_bits(rows.cpu().numpy(), sgo.rows(W, 2), "rows")
     with pytest.raises(ValueError, match="bytes"):
         sg.main(common + ["--iter", "1", "--vector-size", "32", "--init-param-file", str(tmp_path / "one.bin")])
 
@@ -161,7 +162,7 @@ def test_model_rows_and_header(tmp_path, model):
     first = open(tmp_path / "v.txt").readline().split()
     assert first == [str(V + 1), str(14 if model == 0 else 6)]
     _, rows = read_vectors(str(tmp_path / "v.txt"))
-    np.testing.assert_array_equal(rows.cpu().numpy(), sgo.rows(W, model))
+    assert_bits(rows.cpu().numpy(), sgo.rows(W, model), "rows")
     sg.main(["--input-file", path, "--vocab-file", str(vocab), "--vector-size", "6", "--iter", "1", "--model", str(model),
              "--no-unk-vector", "--save-file", str(tmp_path / "n")])
     assert sum(1 for _ in open(tmp_path / "n.txt")) == V
@@ -188,7 +189,7 @@ def test_corpus_to_stanford_glove_to_evaluation(tmp_path, capsys):
     state = sg.StanfordGlove(str(dest / "cooccurrence.shuf.bin"), len(tokens), 20)
     for _ in range(6):
         state.epoch()
-    np.testing.assert_array_equal(rows.cpu().numpy(), state.rows(2, True).cpu().numpy())
+    assert_bits(rows.cpu().numpy(), state.rows(2, True).cpu().numpy(), "rows")
     sf = tmp_path / "s.txt"
     sf.write_text("w0 w1 1.0\nw2 w3 2.0\nw1 w4 3.0\n", encoding="utf8")
     rep = ev.main(["--vectors-txt", out + ".txt", "--similarity", str(sf), "--output-json", str(tmp_path / "r.json")])
